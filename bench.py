@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- BASELINE.json metric: V-cycle ms & HBM GB/s (fraction of peak) at N=16384^2.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Own arm.  Workload = BASELINE.json configs[2] (SURVEY.md 8d "C3"): N=16384, nu=-4e-4, vscale=1,
@@ -20,6 +20,9 @@ towers' HBM allocation is reused between calls of the same shape; the first call
 `--impl reference` times the reference's own CPU implementation (oracle/_ref/libmgref_O3.so: the
 unmodified gs.cpp + multigrid.cpp, run inside an OpenMP team as multigrid.cpp:252-258 does) on a
 bounded sample of the same workload.
+
+`--dump-outputs DIR` writes the field and the residual history the last timed step left (dump_outputs).  The inputs
+depend only on the arguments, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -33,6 +36,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the benchmark writes nothing into the tree it runs from, bytecode caches included
 
 N_FULL = 16384
 NU, VSCALE, TOL = -4e-4, 1.0, 1e-6
@@ -244,6 +248,32 @@ def parity_block(mg, s, n, rank, world, dist, arith_name):
     return out, ok
 
 
+DUMP_U_BYTES = 32 << 20
+
+
+def dump_outputs(out_dir, s, infos, n, rank, world, dist):
+    """--dump-outputs: what the timed steps hand back to a caller, after the last of them, as <out_dir>/<name>.npy
+    (float64), so that two builds run with the same arguments can be compared output for output.
+      u.npy                 the field uT: every row when the field fits in DUMP_U_BYTES, otherwise that many bytes of
+                            whole rows drawn by a fixed seed (the same rows for every run at this N), in row order
+      residual_history.npy  ||r0|| and the residual norm after each V-cycle of the last time step"""
+    import numpy as np
+    nrows = min(n + 1, DUMP_U_BYTES // ((n + 1) * 8))
+    rows = np.arange(n + 1) if nrows == n + 1 else np.sort(np.random.default_rng(0).choice(n + 1, nrows, replace=False))
+    lo, hi, u = s.get_u_host_rows()                     # the rows this rank owns (all rows on one GPU)
+    parts = [u[rows[(rows >= lo) & (rows <= hi)] - lo]]
+    del u
+    if world > 1:
+        mine = parts[0]
+        parts = [None] * world if rank == 0 else None
+        dist.gather_object(mine, parts, dst=0)          # rank r owns the r-th slab of rows: rank order is row order
+    if rank != 0:
+        return
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "u.npy"), np.concatenate(parts, axis=0))
+    np.save(os.path.join(out_dir, "residual_history.npy"), np.array(infos[-1].history(), dtype=np.float64))
+
+
 # ---------------------------------------------------------------------------------------------
 def run_own(args, rank, world):
     import torch
@@ -291,6 +321,8 @@ def run_own(args, rank, world):
         ev1.record(ext)
         ev1.synchronize()
     barrier()
+    if args.dump_outputs:                               # before the measurements below move the field on
+        dump_outputs(args.dump_outputs, s, infos, n, rank, world, dist)
     ms_total = ev0.elapsed_time(ev1)
     if dist:
         t = torch.tensor([ms_total], device="cuda", dtype=torch.float64)
@@ -447,7 +479,13 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-parity", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the field and residual history of the last timed step "
+                    "to DIR/*.npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "own":
+        ap.error("--dump-outputs needs --impl own")
     args.warmup = max(args.warmup, 3) if args.impl == "own" else args.warmup
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))

@@ -14,6 +14,7 @@ SRC = [os.path.join(EMU_DIR, "syst_emu.cpp"),
        os.path.join(ROOT, "hpcclassmultigridproject_b200", "csrc", "syst_pass_body.cuh"),
        os.path.join(ROOT, "hpcclassmultigridproject_b200", "csrc", "common.cuh")]
 SO = os.path.join(EMU_DIR, "libsystemu.so")
+CUDA_INCLUDE = os.path.join(os.environ.get("CUDA_HOME") or "/usr/local/cuda", "include")    # cuda_runtime.h (vector types)
 
 
 def env_without_cc():
@@ -28,8 +29,12 @@ def stale(out, extra=()):
 def load_model():
     """build (if stale) and load the host model of the kernel"""
     if stale(SO):
+        # built under a name of this process and renamed into place: test processes running side by side (pytest -n)
+        # may build it at the same time, and none may load a half-written file
+        tmp = SO[: -len(".so")] + f".{os.getpid()}.so"
         subprocess.run(["g++", "-O2", "-ffp-contract=off", "-std=c++17", "-fPIC", "-shared", "-pthread",
-                        "-I/usr/local/cuda/include", "-o", SO, SRC[0]], check=True, env=env_without_cc())
+                        "-I" + CUDA_INCLUDE, "-o", tmp, SRC[0]], check=True, env=env_without_cc())
+        os.replace(tmp, SO)
     lib = C.CDLL(SO)
     lib.syst_emu_run.restype = C.c_long
     lib.syst_emu_run.argtypes = [C.c_long] * 5 + [_dp] * 8 + [C.c_int] * 3 + [C.c_double] * 3 + [C.c_int] * 3 + [C.c_long] * 6

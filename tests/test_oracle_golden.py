@@ -1,6 +1,8 @@
 """The oracle restatement (oracle/mg_oracle.c) against every known answer we hold:
 golden vectors generated from the compiled reference (tests/golden/make_golden.py) and the
 stdout of the reference's own print tests.  Bit-for-bit wherever the data is binary."""
+import json
+import math
 import os
 import re
 
@@ -31,6 +33,12 @@ SOLVES = ["solve_n32", "solve_n64", "solve_n128", "solve_n256", "solve_cfg_wcycl
           "solve_cfg_n1024"]
 
 
+def exact_norm(a):
+    """||a||_2 from the correctly rounded sum of the squares: the same bits on every host, unlike np.linalg.norm,
+    whose summation order follows the BLAS kernel and its thread count"""
+    return math.sqrt(math.fsum(np.square(a).ravel()))
+
+
 @pytest.mark.parametrize("tag", SOLVES)
 def test_time_steps_bitwise(oracle, tag):
     g = golden(tag + ".npz")
@@ -44,7 +52,13 @@ def test_time_steps_bitwise(oracle, tag):
         assert it == int(g["cycles"][k])
         assert np.array_equal(hist, g["hist"][k][: it + 1])      # norms bit-for-bit (same serial sum)
     uT = s.u(0)
-    assert float(np.linalg.norm(uT)) == float(g["norm_uT"])
+    # the npz's norm_uT carries the rounding of the BLAS that computed it.  With a stored field the norm is taken from
+    # it (the array_equal below already implies this check); without one, from tests/golden/make_golden_norms.py
+    if "uT" in g:
+        want_norm = exact_norm(g["uT"])
+    else:
+        want_norm = json.load(open(os.path.join(GOLDEN, "solve_norms.json")))[tag]
+    assert exact_norm(uT) == want_norm
     assert uT[n // 2, n // 2] == float(g["mid"])
     if "uT" in g:
         assert np.array_equal(uT, g["uT"])

@@ -10,7 +10,7 @@ import subprocess
 import numpy as np
 import pytest
 
-from emu_util import EMU_DIR, SRC, env_without_cc, fields, from_split, layout, load_model, ptr, stale, to_split
+from emu_util import CUDA_INCLUDE, EMU_DIR, SRC, env_without_cc, fields, from_split, layout, load_model, ptr, stale, to_split
 
 
 @pytest.fixture(scope="module")
@@ -172,7 +172,7 @@ def test_barrier_protocol_under_thread_sanitizer():
     main = os.path.join(EMU_DIR, "syst_tsan_main.cpp")
     if stale(exe, [main]):
         r = subprocess.run(["g++", "-O1", "-g", "-fsanitize=thread", "-ffp-contract=off", "-std=c++17", "-pthread",
-                            "-I/usr/local/cuda/include", "-o", exe, main, SRC[0]], capture_output=True, text=True, env=env_without_cc())
+                            "-I" + CUDA_INCLUDE, "-o", exe, main, SRC[0]], capture_output=True, text=True, env=env_without_cc())
         assert r.returncode == 0, r.stderr[-3000:]
     env = dict(env_without_cc(), TSAN_OPTIONS="halt_on_error=0 report_signal_unsafe=0 history_size=4")
     r = subprocess.run([exe], capture_output=True, text=True, env=env, timeout=1700)
