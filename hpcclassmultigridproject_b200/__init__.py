@@ -8,6 +8,7 @@ or CPU implementation of the path, and importing the binding fails loudly when t
 missing.
 """
 from .api import (  # noqa: F401
-    comm_unique_id, default_options, slab_plan, ARITH_EXACT, ARITH_FAST, PLAN_FUSED, PLAN_UNFUSED, MgError, Options, SolveInfo, Solver, lib, maxlvl_for, ops,
+    comm_unique_id, default_options, slab_plan, ARITH_EXACT, ARITH_FAST, PLAN_FUSED, PLAN_UNFUSED, RESTRICT_INJECT,
+    RESTRICT_FW_UNFUSED, RESTRICT_FW, MgError, Options, SolveInfo, Solver, lib, maxlvl_for, ops,
     release_cached, timestepper_device, timestepper_host,
 )

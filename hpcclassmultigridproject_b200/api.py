@@ -11,6 +11,8 @@ LIB_PATH = os.environ.get("MGB200_LIB") or os.path.join(HERE, "libmgb200.so")   
 
 ARITH_FAST, ARITH_EXACT = 0, 1
 PLAN_FUSED, PLAN_UNFUSED = 0, 1
+# Options.restriction: injection (the reference), full weighting on the UNFUSED plan only, full weighting on either plan
+RESTRICT_INJECT, RESTRICT_FW_UNFUSED, RESTRICT_FW = 0, 1, 2
 
 
 class MgError(RuntimeError):

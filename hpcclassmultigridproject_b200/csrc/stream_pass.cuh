@@ -13,7 +13,9 @@ namespace mgb200 {
 enum StreamPost {
     POST_NONE = 0,
     POST_INJECT = 1,   // coarse_rhs[I][J] = residual(2I,2J) on the coarse interior (residual ; restriction)
-    POST_NORM2 = 2     // sum of squares of the residual over the interior -> partials (residual ; compute_norm)
+    POST_NORM2 = 2,    // sum of squares of the residual over the interior -> partials (residual ; compute_norm)
+    POST_FW = 3        // coarse_rhs[I][J] = full weighting of the residual on the coarse interior (residual ;
+                       // restriction_fw); down leg only (no prolongation in the same pass)
 };
 
 struct StreamPassArgs {
@@ -31,7 +33,7 @@ struct StreamPassArgs {
     Layout Lc;              // layout of the (n/2) level
     // optional epilogue
     int post;               // StreamPost
-    double* coarse_rhs;     // POST_INJECT target (layout Lc)
+    double* coarse_rhs;     // POST_INJECT / POST_FW target (layout Lc)
     double* partials;       // POST_NORM2: one double per tile, stream_pass_tiles() entries
     int arith;
     // row window (row-slab sharding).  rows_mem == 0 means "whole level": rows 0..n owned and held.
@@ -39,7 +41,7 @@ struct StreamPassArgs {
     long row0, rows_mem;    // fine arrays hold global rows row0 .. row0+rows_mem-1
     long crow0, crows_mem;  // same for the coarse arrays
     // Halo push fused into the pass (row slabs over NVLink peer memory; all null / 0 otherwise).  The pass stores
-    // the first / last `push_rows` rows it produces (and the matching rows of the coarse rhs of a POST_INJECT
+    // the first / last `push_rows` rows it produces (and the matching rows of the coarse rhs of a POST_INJECT / POST_FW
     // pass whose child level is sharded too) straight into the slab neighbours' halo rows, raises their arrival
     // counters when it ends and, at its start, lets only the tiles that stage halo rows wait for the
     // neighbours' previous pass.  peer_*: the neighbours' copies of u_out / coarse_rhs, addressed like ours

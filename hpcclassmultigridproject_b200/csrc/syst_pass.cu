@@ -150,7 +150,7 @@ __global__ void __launch_bounds__(THREADS, 1) k_syst_pass(const __grid_constant_
     Smem sm;
     carve(sm, smem_raw, p.SWK);
     sm.base32 = smem_u32(smem_raw);
-    const Tile tl = make_tile(p, blockIdx.x);
+    const Tile tl = make_tile(p, blockIdx.x, POSTK == POST_FW ? 1 : 0);
     const Geo geo = make_geo(p);
     // warp index through a shuffle: provably warp-uniform, so that role branches are uniform and
     // the load and store warps' operands live in uniform registers
@@ -242,6 +242,8 @@ static PassKernel pass_kernel_of(bool pre, int post)
 }
 static PassKernel pass_kernel(int arith, bool pre, int post)
 {
+    // full weighting: down leg only, no prolongation flavour
+    if (post == POST_FW) return arith == MGB200_ARITH_EXACT ? k_syst_pass<MGB200_ARITH_EXACT, false, POST_FW> : k_syst_pass<MGB200_ARITH_FAST, false, POST_FW>;
     return arith == MGB200_ARITH_EXACT ? pass_kernel_of<MGB200_ARITH_EXACT>(pre, post) : pass_kernel_of<MGB200_ARITH_FAST>(pre, post);
 }
 
@@ -263,6 +265,8 @@ int stream_pass_init()
         for (int pre = 0; pre < 2; ++pre)
             for (int post = 0; post < 3; ++post)
                 MGB_CUDA(cudaFuncSetAttribute(pass_kernel(arith, pre != 0, post), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_BYTES));
+    for (int arith = 0; arith < 2; ++arith)
+        MGB_CUDA(cudaFuncSetAttribute(pass_kernel(arith, false, POST_FW), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_BYTES));
     if (!g_encode) {
         void* fn = nullptr;
         cudaDriverEntryPointQueryResult qres;
@@ -325,6 +329,7 @@ static int build_params(const StreamPassArgs& a, Params& p, unsigned& grid_out, 
     p.push_rows = a.push_rows; p.c_own_lo = a.c_own_lo; p.c_own_hi = a.c_own_hi;
     p.sync = a.sync; p.raise_up = a.raise_up; p.raise_dn = a.raise_dn;
     if (p.post == POST_INJECT && !p.crhs) return fail(MGB200_ERR_INVALID, "stream_pass: POST_INJECT without coarse_rhs");
+    if (p.post == POST_FW && (!p.crhs || p.pre)) return fail(MGB200_ERR_INVALID, "stream_pass: POST_FW needs coarse_rhs and no prolongation");
     if (p.post == POST_NORM2 && !p.partials) return fail(MGB200_ERR_INVALID, "stream_pass: POST_NORM2 without partials");
     grid_out = (unsigned)(pl.nstrips * pl.nbands);
     smem_out = smem_bytes(pl.SWK);

@@ -6,7 +6,7 @@
 //
 //   multigrid_b200 [--N 256] [--steps 100] [--nu -4e-4] [--vscale 1] [--tol 1e-6] [--shape 1]
 //                  [--niter 3] [--coarse-tol 1e-5] [--coarse-maxit 1000] [--max-cycle 50]     (multigrid.cpp:41,60,94)
-//                  [--correct-towers] [--exact] [--unfused] [--gpus 1]
+//                  [--correct-towers] [--exact] [--unfused] [--full-weighting] [--gpus 1]
 //                  [--out uT.txt] [--bin uT.f64] [--quiet]
 // --gpus P > 1: the program forks P processes, one per GPU (row slabs, include/mgb200.h "Row-slab sharding");
 // process 0 creates the communicator id and hands it to the others through pipes, every process writes the rows
@@ -88,6 +88,7 @@ int main(int argc, char** argv)
         else if (k == "--gpus") gpus = std::atoi(val());
         else if (k == "--exact") opt.arith = MGB200_ARITH_EXACT;
         else if (k == "--unfused") opt.plan = MGB200_PLAN_UNFUSED;
+        else if (k == "--full-weighting") opt.restriction = MGB200_RESTRICT_FW;
         else if (k == "--out") out = val();
         else if (k == "--bin") bin = val();
         else if (k == "--quiet") quiet = true;
