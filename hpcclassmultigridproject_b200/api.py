@@ -65,6 +65,8 @@ def lib():
     L.mgb200_default_options.argtypes = [C.POINTER(Options)]
     L.mgb200_default_options.restype = None
     L.mgb200_create.argtypes = [C.POINTER(_vp), _l, _i, _d, _d, _d, _d, C.POINTER(Options)]
+    L.mgb200_create_batched.argtypes = [C.POINTER(_vp), _l, _i, _i, _d, _d, _d, _d, C.POINTER(Options)]
+    L.mgb200_batch_size.argtypes = [_vp]; L.mgb200_batch_size.restype = _i
     L.mgb200_comm_unique_id.argtypes = [C.c_char_p]
     L.mgb200_create_sharded.argtypes = [C.POINTER(_vp), _l, _i, _d, _d, _d, _d, C.POINTER(Options), _i, _i, C.c_char_p, _l]
     L.mgb200_slab.argtypes = [_vp, _i, C.POINTER(_l * 6)]
@@ -201,16 +203,24 @@ ops = _Ops()
 
 
 class Solver:
-    """mgb200_solver handle: the V/W-cycle driver (mg_inner / mg_outer / timestepper)."""
+    """mgb200_solver handle: the V/W-cycle driver (mg_inner / mg_outer / timestepper).
 
-    def __init__(self, n, nu, dt, dx, tol, maxlvl=None, rank=0, nranks=1, unique_id=None, shard_min_rows=0, **opts):
+    batch=B: a batched handle of B independent problems of this size (mgb200_create_batched).  Fields are then
+    (B, n+1, n+1) arrays; form_rhs / cycle / last_norm return B norms, solve B infos, timestep a list of nsteps lists
+    of B infos, get_u_host / level (B, n+1, n+1) arrays."""
+
+    def __init__(self, n, nu, dt, dx, tol, maxlvl=None, rank=0, nranks=1, unique_id=None, shard_min_rows=0, batch=None, **opts):
         """nranks > 1: row-slab sharded handle (one process per GPU); unique_id = comm_unique_id() of rank 0"""
         self.n = n
         self.maxlvl = maxlvl_for(n) if maxlvl is None else maxlvl
         self.opt = default_options(**opts)
         self.rank, self.nranks = rank, nranks
+        self.batch = batch
         self.h = _vp()
-        if nranks == 1:
+        if batch is not None:
+            assert nranks == 1, "batched handles run on one GPU"
+            _ck(lib().mgb200_create_batched(C.byref(self.h), n, self.maxlvl, batch, nu, dt, dx, tol, C.byref(self.opt)))
+        elif nranks == 1:
             _ck(lib().mgb200_create(C.byref(self.h), n, self.maxlvl, nu, dt, dx, tol, C.byref(self.opt)))
         else:
             assert unique_id is not None and len(unique_id) == 128
@@ -239,48 +249,70 @@ class Solver:
     def __exit__(self, *a):
         self.close()
 
+    @property
+    def members(self) -> int:
+        """problems the handle holds (1 unless batched)"""
+        return lib().mgb200_batch_size(self.h)
+
+    def _shape(self, nl):
+        return (nl + 1, nl + 1) if self.batch is None else (self.batch, nl + 1, nl + 1)
+
+    def _norms(self, fn):
+        r = (_d * self.members)()
+        _ck(fn(self.h, r))
+        return r[0] if self.batch is None else list(r)
+
     def set_fields_device(self, u0, v1, v2):
+        if self.batch is not None:
+            for a in (u0, v1, v2):
+                assert tuple(a.shape) == self._shape(self.n) and a.stride(0) == (self.n + 1) * a.stride(1), "members (n+1) rows apart"
+            _ck(lib().mgb200_set_fields_device(self.h, _ptr(u0), _ptr(v1), _ptr(v2), u0.stride(1)))
+            return
         _ck(lib().mgb200_set_fields_device(self.h, _ptr(u0), _ptr(v1), _ptr(v2), u0.stride(0)))
 
     def set_fields_host(self, u0, v1, v2):
-        """numpy arrays or pinned torch CPU tensors, dense (n+1)^2"""
+        """numpy arrays or pinned torch CPU tensors, dense (n+1)^2 (batched: dense (B, n+1, n+1))"""
+        if self.batch is not None:
+            for a in (u0, v1, v2):
+                assert tuple(a.shape) == self._shape(self.n), (tuple(a.shape), self._shape(self.n))
+                assert a.flags["C_CONTIGUOUS"] if hasattr(a, "flags") else a.is_contiguous()
         _ck(lib().mgb200_set_fields_host(self.h, _ptr(u0), _ptr(v1), _ptr(v2)))
 
     def set_fields_reference_ic(self, vscale=1.0):
         _ck(lib().mgb200_set_fields_reference_ic(self.h, vscale))
 
-    def form_rhs(self) -> float:
-        r = _d(0.0)
-        _ck(lib().mgb200_form_rhs(self.h, C.byref(r)))
-        return r.value
+    def form_rhs(self):
+        return self._norms(lib().mgb200_form_rhs)
 
-    def cycle(self) -> float:
-        r = _d(0.0)
-        _ck(lib().mgb200_cycle(self.h, C.byref(r)))
-        return r.value
+    def cycle(self):
+        return self._norms(lib().mgb200_cycle)
 
     def cycle_async(self):
         _ck(lib().mgb200_cycle_async(self.h))
 
-    def last_norm(self) -> float:
-        r = _d(0.0)
-        _ck(lib().mgb200_last_norm(self.h, C.byref(r)))
-        return r.value
+    def last_norm(self):
+        return self._norms(lib().mgb200_last_norm)
 
-    def solve(self) -> SolveInfo:
-        info = SolveInfo()
-        _ck(lib().mgb200_solve(self.h, C.byref(info)))
-        return info
+    def solve(self):
+        """SolveInfo (batched: a list of B)"""
+        infos = (SolveInfo * self.members)()
+        _ck(lib().mgb200_solve(self.h, infos))
+        return infos[0] if self.batch is None else list(infos)
 
     def timestep(self, nsteps):
-        infos = (SolveInfo * nsteps)()
+        """nsteps SolveInfos (batched: nsteps lists of B)"""
+        B = self.members
+        infos = (SolveInfo * (nsteps * B))()
         _ck(lib().mgb200_timestep(self.h, nsteps, infos))
-        return list(infos)
+        if self.batch is None:
+            return list(infos)
+        return [list(infos[k * B:(k + 1) * B]) for k in range(nsteps)]
 
     def get_u_host(self, out=None):
         import numpy as np
         if out is None:
-            out = np.full((self.n + 1, self.n + 1), np.nan) if self.nranks > 1 else np.empty((self.n + 1, self.n + 1))
+            out = np.full(self._shape(self.n), np.nan) if self.nranks > 1 else np.empty(self._shape(self.n))
+        assert out.shape == self._shape(self.n) and out.flags["C_CONTIGUOUS"]
         _ck(lib().mgb200_get_u_host(self.h, _ptr(out)))
         return out
 
@@ -307,6 +339,10 @@ class Solver:
         return lo, hi, out
 
     def get_u_device(self, out):
+        if self.batch is not None:
+            assert tuple(out.shape) == self._shape(self.n) and out.stride(0) == (self.n + 1) * out.stride(1)
+            _ck(lib().mgb200_get_u_device(self.h, _ptr(out), out.stride(1)))
+            return out
         _ck(lib().mgb200_get_u_device(self.h, _ptr(out), out.stride(0)))
         return out
 
@@ -314,7 +350,7 @@ class Solver:
         """dense copy of a level array; a slab rank fills only the rows it holds (the rest is NaN)"""
         import numpy as np
         nl = self.n >> lvl
-        out = np.full((nl + 1, nl + 1), np.nan)
+        out = np.full(self._shape(nl), np.nan)
         _ck(lib().mgb200_get_level_host(self.h, lvl, {"u": 0, "rhs": 1, "v1": 2, "v2": 3}[which], _ptr(out)))
         return out
 

@@ -106,10 +106,10 @@ __global__ void __launch_bounds__(TPB) k_compute_rhs(double* __restrict__ rhs, c
 // lanes come from shuffles.  Same operands in the same order as k_compute_rhs: identical rhs.
 constexpr int RHS_TPB = 128, RHS_ROWS = 32;
 template <int ARITH, bool WITH_RES0>
-__global__ void __launch_bounds__(RHS_TPB) k_compute_rhs_split(double* __restrict__ rhs, const double* __restrict__ u,
-                                                               const double* __restrict__ v1, const double* __restrict__ v2,
-                                                               long n, Layout L, Stencil st, double* __restrict__ partials,
-                                                               long ilo, long ihi)
+__device__ __forceinline__ void compute_rhs_split_body(double* __restrict__ rhs, const double* __restrict__ u,
+                                                       const double* __restrict__ v1, const double* __restrict__ v2,
+                                                       long n, Layout L, Stencil st, double* __restrict__ partials,
+                                                       long ilo, long ihi)
 {
     __shared__ double scratch[32];
     const int lane = threadIdx.x & 31;
@@ -158,6 +158,27 @@ __global__ void __launch_bounds__(RHS_TPB) k_compute_rhs_split(double* __restric
     }
 }
 
+template <int ARITH, bool WITH_RES0>
+__global__ void __launch_bounds__(RHS_TPB) k_compute_rhs_split(double* __restrict__ rhs, const double* __restrict__ u,
+                                                               const double* __restrict__ v1, const double* __restrict__ v2,
+                                                               long n, Layout L, Stencil st, double* __restrict__ partials,
+                                                               long ilo, long ihi)
+{
+    compute_rhs_split_body<ARITH, WITH_RES0>(rhs, u, v1, v2, n, L, st, partials, ilo, ihi);
+}
+
+// a batch of problems (batched solver handles): member blockIdx.z at + blockIdx.z * mstride in every field, its
+// partial sums at + blockIdx.z * pstride, each member's in the order of k_compute_rhs_split
+template <int ARITH>
+__global__ void __launch_bounds__(RHS_TPB) k_compute_rhs_split_batched(double* __restrict__ rhs, const double* __restrict__ u,
+                                                                       const double* __restrict__ v1, const double* __restrict__ v2,
+                                                                       long n, Layout L, Stencil st, double* __restrict__ partials,
+                                                                       long ilo, long ihi, long mstride, long pstride)
+{
+    const long mo = (long)blockIdx.z * mstride;
+    compute_rhs_split_body<ARITH, true>(rhs + mo, u + mo, v1 + mo, v2 + mo, n, L, st, partials + (long)blockIdx.z * pstride, ilo, ihi);
+}
+
 __global__ void __launch_bounds__(TPB) k_square_partials(const double* __restrict__ a, long n, Layout L,
                                                          double* __restrict__ partials)
 {
@@ -183,6 +204,19 @@ __global__ void __launch_bounds__(1024) k_reduce_partials(const double* __restri
     for (long q = threadIdx.x; q < count; q += 1024) acc += partials[q];
     const double t = block_sum(acc, scratch);
     if (threadIdx.x == 0) out[0] = t;
+}
+
+// one block per member, each summing in the order of k_reduce_partials; active == null: every member
+__global__ void __launch_bounds__(1024) k_reduce_partials_batched(const double* __restrict__ partials, long count, long pstride,
+                                                                  double* __restrict__ out, const int* __restrict__ active)
+{
+    __shared__ double scratch[32];
+    if (active && !active[blockIdx.x]) return;
+    const double* part = partials + (long)blockIdx.x * pstride;
+    double acc = 0.0;
+    for (long q = threadIdx.x; q < count; q += 1024) acc += part[q];
+    const double t = block_sum(acc, scratch);
+    if (threadIdx.x == 0) out[blockIdx.x] = t;
 }
 
 template <bool INTERIOR>
@@ -336,10 +370,10 @@ __global__ void __launch_bounds__(TPB) k_flat_to_level(double* __restrict__ dst,
 // ---------------------------------------------------------------------------------------------
 // Coarsest level on ONE thread block, all fields staged in shared memory (natural order).
 template <int ARITH>
-__global__ void __launch_bounds__(1024) k_coarse_solve(double* __restrict__ u, const double* __restrict__ rhs,
-                                                       const double* __restrict__ v1, const double* __restrict__ v2,
-                                                       int n, Layout L, Stencil st, int zero_init, int maxit,
-                                                       double tol, int* __restrict__ iters_out)
+__device__ __forceinline__ void coarse_solve_body(double* __restrict__ u, const double* __restrict__ rhs,
+                                                  const double* __restrict__ v1, const double* __restrict__ v2,
+                                                  int n, Layout L, Stencil st, int zero_init, int maxit,
+                                                  double tol, int* __restrict__ iters_out)
 {
     extern __shared__ double sm[];
     __shared__ double scratch[32];
@@ -399,6 +433,29 @@ __global__ void __launch_bounds__(1024) k_coarse_solve(double* __restrict__ u, c
     if (threadIdx.x == 0 && iters_out) *iters_out = it;
 }
 
+template <int ARITH>
+__global__ void __launch_bounds__(1024) k_coarse_solve(double* __restrict__ u, const double* __restrict__ rhs,
+                                                       const double* __restrict__ v1, const double* __restrict__ v2,
+                                                       int n, Layout L, Stencil st, int zero_init, int maxit,
+                                                       double tol, int* __restrict__ iters_out)
+{
+    coarse_solve_body<ARITH>(u, rhs, v1, v2, n, L, st, zero_init, maxit, tol, iters_out);
+}
+
+// one block per member (blockIdx.x, fields mstride apart); a frozen member (active == 0) is left as it is
+template <int ARITH>
+__global__ void __launch_bounds__(1024) k_coarse_solve_batched(double* __restrict__ u, const double* __restrict__ rhs,
+                                                               const double* __restrict__ v1, const double* __restrict__ v2,
+                                                               int n, Layout L, Stencil st, int zero_init, int maxit,
+                                                               double tol, int* __restrict__ iters_out, long mstride,
+                                                               const int* __restrict__ active)
+{
+    const int b = blockIdx.x;
+    if (!active[b]) return;
+    const long mo = (long)b * mstride;
+    coarse_solve_body<ARITH>(u + mo, rhs + mo, v1 + mo, v2 + mo, n, L, st, zero_init, maxit, tol, iters_out + b);
+}
+
 // ---- opt-in direct solve of the coarsest level (the unfinished exact_solve.cpp:1-55 of the reference) -------------
 // Unknowns: the (n-1)^2 interior nodes, p = (i-1)(n-1) + (j-1); half bandwidth w = n-1; band storage
 // AB[p][w + q - p] for |q - p| <= w (row p of A, (2w+1) doubles per row).  LU without pivoting (A is strictly
@@ -454,9 +511,9 @@ __global__ void __launch_bounds__(1024) k_coarse_lu_factor(double* __restrict__ 
 
 // u(interior) = A^-1 (rhs - boundary terms): forward substitution with the stored multipliers, back substitution
 // with U.  y lives in shared memory.
-__global__ void __launch_bounds__(128) k_coarse_lu_solve(double* __restrict__ u, const double* __restrict__ rhs,
-                                                         const double* __restrict__ v1, const double* __restrict__ v2,
-                                                         const double* __restrict__ ab, int n, Layout L, Stencil st, int zero_init)
+__device__ __forceinline__ void coarse_lu_solve_body(double* __restrict__ u, const double* __restrict__ rhs,
+                                                     const double* __restrict__ v1, const double* __restrict__ v2,
+                                                     const double* __restrict__ ab, int n, Layout L, Stencil st, int zero_init)
 {
     extern __shared__ double y[];
     const int ni = n - 1, m = ni * ni, w = ni, bw = 2 * w + 1;
@@ -494,6 +551,26 @@ __global__ void __launch_bounds__(128) k_coarse_lu_solve(double* __restrict__ u,
     for (int p = threadIdx.x; p < m; p += blockDim.x) u[L.at(1 + p / ni, 1 + p % ni)] = y[p];
 }
 
+__global__ void __launch_bounds__(128) k_coarse_lu_solve(double* __restrict__ u, const double* __restrict__ rhs,
+                                                         const double* __restrict__ v1, const double* __restrict__ v2,
+                                                         const double* __restrict__ ab, int n, Layout L, Stencil st, int zero_init)
+{
+    coarse_lu_solve_body(u, rhs, v1, v2, ab, n, L, st, zero_init);
+}
+
+// one block per member: fields mstride apart, factors abstride apart; a frozen member is left as it is
+__global__ void __launch_bounds__(128) k_coarse_lu_solve_batched(double* __restrict__ u, const double* __restrict__ rhs,
+                                                                 const double* __restrict__ v1, const double* __restrict__ v2,
+                                                                 const double* __restrict__ ab, int n, Layout L, Stencil st,
+                                                                 int zero_init, long mstride, long abstride,
+                                                                 const int* __restrict__ active)
+{
+    const int b = blockIdx.x;
+    if (!active[b]) return;
+    const long mo = (long)b * mstride;
+    coarse_lu_solve_body(u + mo, rhs + mo, v1 + mo, v2 + mo, ab + (long)b * abstride, n, L, st, zero_init);
+}
+
 }  // namespace
 
 int ops_basic_init()
@@ -508,6 +585,8 @@ int ops_basic_init()
     const int smem = 4 * 65 * 65 * (int)sizeof(double);
     MGB_CUDA(cudaFuncSetAttribute(k_coarse_solve<MGB200_ARITH_EXACT>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
     MGB_CUDA(cudaFuncSetAttribute(k_coarse_solve<MGB200_ARITH_FAST>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    MGB_CUDA(cudaFuncSetAttribute(k_coarse_solve_batched<MGB200_ARITH_EXACT>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    MGB_CUDA(cudaFuncSetAttribute(k_coarse_solve_batched<MGB200_ARITH_FAST>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
     if (dev >= 0 && dev < 64) done[dev] = true;
     return MGB200_OK;
 }
@@ -711,6 +790,56 @@ int launch_coarse_solve(double* u, const double* rhs, const double* v1, const do
         k_coarse_solve<MGB200_ARITH_FAST><<<1, 1024, smem, s>>>(u, rhs, v1, v2, (int)n, L, st, zero_init ? 1 : 0, maxit, tol, iters_out);
     }
     return check_launch("k_coarse_solve");
+}
+
+// ---------------------------------------------------------------------------------------------
+// batched solver handles: `members` problems, member b of every array at + b * mstride
+int launch_compute_rhs_batched(double* rhs, const double* u, const double* v1, const double* v2, long n, Layout L,
+                               const Stencil& st, int arith, double* partials, long pstride, int members, long mstride,
+                               cudaStream_t s)
+{
+    if (!is_split(L, n) || n < 4 || members < 1 || members > 65535) return fail(MGB200_ERR_INVALID, "compute_rhs_batched: bad argument");
+    dim3 g = rhs_split_grid(n, n - 1);
+    if ((long)g.x * g.y > pstride) return fail(MGB200_ERR_INVALID, "compute_rhs_batched: partials stride too small");
+    g.z = (unsigned)members;
+    if (arith == MGB200_ARITH_EXACT)
+        k_compute_rhs_split_batched<MGB200_ARITH_EXACT><<<g, RHS_TPB, 0, s>>>(rhs, u, v1, v2, n, L, st, partials, 1, n - 1, mstride, pstride);
+    else
+        k_compute_rhs_split_batched<MGB200_ARITH_FAST><<<g, RHS_TPB, 0, s>>>(rhs, u, v1, v2, n, L, st, partials, 1, n - 1, mstride, pstride);
+    return check_launch("k_compute_rhs_split_batched");
+}
+
+int launch_reduce_partials_batched(const double* partials, long count, long pstride, double* out, const int* active, int members,
+                                   cudaStream_t s)
+{
+    k_reduce_partials_batched<<<members, 1024, 0, s>>>(partials, count, pstride, out, active);
+    return check_launch("k_reduce_partials_batched");
+}
+
+int launch_coarse_solve_batched(double* u, const double* rhs, const double* v1, const double* v2, long n, Layout L,
+                                const Stencil& st, int arith, bool zero_init, int maxit, double tol, int* iters_out,
+                                int members, long mstride, const int* active, cudaStream_t s)
+{
+    if (n > 64) return fail(MGB200_ERR_INVALID, "coarse_solve: n > 64 not supported by the single-block kernel");
+    const size_t smem = 4 * (size_t)(n + 1) * (n + 1) * sizeof(double);
+    MGB_TRY(ops_basic_init());
+    if (arith == MGB200_ARITH_EXACT)
+        k_coarse_solve_batched<MGB200_ARITH_EXACT><<<members, 1024, smem, s>>>(u, rhs, v1, v2, (int)n, L, st, zero_init ? 1 : 0, maxit, tol,
+                                                                              iters_out, mstride, active);
+    else
+        k_coarse_solve_batched<MGB200_ARITH_FAST><<<members, 1024, smem, s>>>(u, rhs, v1, v2, (int)n, L, st, zero_init ? 1 : 0, maxit, tol,
+                                                                             iters_out, mstride, active);
+    return check_launch("k_coarse_solve_batched");
+}
+
+int launch_coarse_lu_solve_batched(double* u, const double* rhs, const double* v1, const double* v2, const double* ab, long n,
+                                   Layout L, const Stencil& st, bool zero_init, int members, long mstride, long abstride,
+                                   const int* active, cudaStream_t s)
+{
+    if (n > 64 || n < 4) return fail(MGB200_ERR_INVALID, "coarse_lu: 4 <= n <= 64");
+    k_coarse_lu_solve_batched<<<members, 128, (size_t)(n - 1) * (n - 1) * sizeof(double), s>>>(u, rhs, v1, v2, ab, (int)n, L, st,
+                                                                                               zero_init ? 1 : 0, mstride, abstride, active);
+    return check_launch("k_coarse_lu_solve_batched");
 }
 
 }  // namespace mgb200

@@ -65,4 +65,22 @@ int launch_coarse_lu_factor(double* ab, const double* v1, const double* v2, long
 int launch_coarse_lu_solve(double* u, const double* rhs, const double* v1, const double* v2, const double* ab, long n, Layout L,
                            const Stencil& st, bool zero_init, cudaStream_t s);
 
+// Batched solver handles: `members` problems of one size, member b of every field at + b * mstride.
+// rhs = B u and the sum of squares of the initial residual of every member (partials of member b at
+// + b * pstride: compute_rhs_partials_count(n, n - 1, L) each)
+int launch_compute_rhs_batched(double* rhs, const double* u, const double* v1, const double* v2, long n, Layout L,
+                               const Stencil& st, int arith, double* partials, long pstride, int members, long mstride,
+                               cudaStream_t s);
+// out[b] = sum of member b's `count` partials (in launch_reduce_partials' order) for every member with active[b] != 0
+// (active == NULL: every member)
+int launch_reduce_partials_batched(const double* partials, long count, long pstride, double* out, const int* active, int members,
+                                   cudaStream_t s);
+// the coarsest-level solves of the active members, one block each (iters_out[b], factors of member b at + b * abstride)
+int launch_coarse_solve_batched(double* u, const double* rhs, const double* v1, const double* v2, long n, Layout L,
+                                const Stencil& st, int arith, bool zero_init, int maxit, double tol, int* iters_out,
+                                int members, long mstride, const int* active, cudaStream_t s);
+int launch_coarse_lu_solve_batched(double* u, const double* rhs, const double* v1, const double* v2, const double* ab, long n,
+                                   Layout L, const Stencil& st, bool zero_init, int members, long mstride, long abstride,
+                                   const int* active, cudaStream_t s);
+
 }  // namespace mgb200

@@ -128,6 +128,45 @@ __global__ void k_loop_check(cudaGraphConditionalHandle h, const double* norm2, 
     cudaGraphSetConditional(h, (it < st->max_cycle && r / st->res0 > st->tol) ? 1u : 0u);
 }
 
+// Batched handles: the same loop per member (one block, members strided over its threads).  A member runs while its
+// own condition holds; active[b] tells the passes of the next cycle whether to touch member b, and the loop goes on
+// while any member is active.
+__global__ void k_loop_begin_batched(cudaGraphConditionalHandle h, const double* norm2, LoopState* st, int* active, double tol,
+                                     int max_cycle, int members)
+{
+    int any = 0;
+    for (int b = threadIdx.x; b < members; b += blockDim.x) {
+        const double r0 = sqrt(norm2[b]);
+        LoopState& s = st[b];
+        s.res0 = r0; s.tol = tol; s.iter = 0; s.max_cycle = max_cycle; s.hist[0] = r0;
+        const int go = (0 < max_cycle && r0 / r0 > tol) ? 1 : 0;
+        active[b] = go; any |= go;
+    }
+    any = __syncthreads_or(any);
+    if (threadIdx.x == 0) cudaGraphSetConditional(h, any ? 1u : 0u);
+}
+
+__global__ void k_loop_check_batched(cudaGraphConditionalHandle h, const double* norm2, LoopState* st, int* active, int members)
+{
+    int any = 0;
+    for (int b = threadIdx.x; b < members; b += blockDim.x) {
+        if (!active[b]) continue;
+        LoopState& s = st[b];
+        const double r = sqrt(norm2[b]);
+        const int it = ++s.iter;
+        s.hist[it] = r;
+        const int go = (it < s.max_cycle && r / s.res0 > s.tol) ? 1 : 0;
+        active[b] = go; any |= go;
+    }
+    any = __syncthreads_or(any);
+    if (threadIdx.x == 0) cudaGraphSetConditional(h, any ? 1u : 0u);
+}
+
+__global__ void k_fill_int(int* a, int n, int v)
+{
+    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) a[i] = v;
+}
+
 }  // namespace mgb200
 
 using namespace mgb200;
@@ -147,6 +186,20 @@ struct mgb200_solver {
     int* d_coarse_iters = nullptr;
     double* d_coarse_lu = nullptr;     // opt-in direct coarsest solve: the factored band matrix (options.coarse_exact)
     double* d_flat[2] = {nullptr, nullptr};
+    // Batched handle (mgb200_create_batched): `batch` independent problems of this size; member b of every level
+    // array lives at + b * elems of one allocation, its partial sums at d_partials + b * pstride, its norm in
+    // d_norm2[b], its loop state in d_loop[b].  0: a handle of one problem.
+    int batch = 0;
+    long pstride = 0;
+    int* d_active = nullptr;           // per member: 1 while it iterates (a pass leaves a member with 0 untouched)
+    int* h_active = nullptr;           // pinned mirror (host loop)
+    std::vector<double> res0_b, res_b; // per member: host copies of res0 / the last norm
+    int  members() const { return batch > 0 ? batch : 1; }
+    int  activate_all();
+    int  read_norms(double* out);
+    int  solve_batched(mgb200_solve_info* infos);
+    int  timestep_batched(int nsteps, mgb200_solve_info* infos);
+    void fill_pass_batch(StreamPassArgs& a, const Level& g, const Level& c) const;
     cudaGraphExec_t graph_exec = nullptr;
     long graph_kernels = 0;
     // the whole mg_outer loop as one graph: a WHILE node around the cycle, condition set on the device
@@ -255,6 +308,8 @@ void mgb200_solver::release()
     cudaFree(d_norm2); d_norm2 = nullptr;
     cudaFree(d_coarse_iters); d_coarse_iters = nullptr;
     cudaFree(d_coarse_lu); d_coarse_lu = nullptr;
+    cudaFree(d_active); d_active = nullptr;
+    if (h_active) { cudaFreeHost(h_active); h_active = nullptr; }
     cudaFree(d_flat[0]); cudaFree(d_flat[1]); d_flat[0] = d_flat[1] = nullptr;
     for (auto& t : d_top) { cudaFree(t); t = nullptr; }
     cudaFree(d_sync); d_sync = nullptr;
@@ -279,6 +334,11 @@ int mgb200_solver::init(long n, int maxlvl_, double nu_, double dt_, double dx_,
     if (opt.shape < 1 || opt.niter < 0 || opt.max_cycle < 0 || opt.max_cycle > 50)
         return fail(MGB200_ERR_INVALID, "bad options (shape >= 1, niter >= 0, 0 <= max_cycle <= 50)");
     if (opt.coarse_exact != 0 && opt.coarse_exact != 1) return fail(MGB200_ERR_INVALID, "options.coarse_exact: 0 or 1");
+    if (batch > 0) {
+        if (batch > STREAM_PASS_MAX_MEMBERS) return fail(MGB200_ERR_INVALID, "batch: at most 65535 members (gridDim.y of the batched pass)");
+        if (opt.plan != MGB200_PLAN_FUSED) return fail(MGB200_ERR_INVALID, "a batched handle runs the fused plan only (options.plan = 0)");
+        if (opt.niter == 0) return fail(MGB200_ERR_INVALID, "a batched handle needs niter >= 1 (niter = 0 implies the unfused plan)");
+    }
     if (opt.restriction != MGB200_RESTRICT_INJECT && opt.restriction != MGB200_RESTRICT_FW &&
         (opt.restriction != MGB200_RESTRICT_FW_UNFUSED || opt.plan != MGB200_PLAN_UNFUSED))
         return fail(MGB200_ERR_INVALID, "options.restriction: 0 (injection), 1 (full weighting, UNFUSED plan only) or 2 (full weighting)");
@@ -310,15 +370,28 @@ int mgb200_solver::init(long n, int maxlvl_, double nu_, double dt_, double dx_,
     MGB_TRY(ops_basic_init());
     if (opt.plan == MGB200_PLAN_FUSED) MGB_TRY(stream_pass_init());
     MGB_TRY(alloc_levels());
-    partials_cap = std::max(residual_partials_count(N), stream_pass_tiles(N, lv[0].own_hi - lv[0].own_lo + 1, -1)) + 8;
+    if (batch == 0) {
+        partials_cap = std::max(residual_partials_count(N), stream_pass_tiles(N, lv[0].own_hi - lv[0].own_lo + 1, -1)) + 8;
+    } else {
+        pstride = std::max(std::max(residual_partials_count(N), compute_rhs_partials_count(N, N - 1, lv[0].L)),
+                           stream_pass_tiles(N, N + 1, -1, batch)) + 8;
+        partials_cap = pstride * batch;
+    }
+    const size_t mb = (size_t)members();
     MGB_CUDA(cudaMalloc(&d_partials, partials_cap * sizeof(double)));
-    MGB_CUDA(cudaMalloc(&d_norm2, 8 * sizeof(double)));
-    MGB_CUDA(cudaMemsetAsync(d_norm2, 0, 8 * sizeof(double), stream));
-    MGB_CUDA(cudaMalloc(&d_coarse_iters, sizeof(int)));
-    MGB_CUDA(cudaMallocHost(&h_norm2, 8 * sizeof(double)));
-    MGB_CUDA(cudaMalloc(&d_loop, sizeof(LoopState)));
-    MGB_CUDA(cudaMemsetAsync(d_loop, 0, sizeof(LoopState), stream));
-    MGB_CUDA(cudaMallocHost(&h_loop, sizeof(LoopState)));
+    MGB_CUDA(cudaMalloc(&d_norm2, (8 + mb) * sizeof(double)));
+    MGB_CUDA(cudaMemsetAsync(d_norm2, 0, (8 + mb) * sizeof(double), stream));
+    MGB_CUDA(cudaMalloc(&d_coarse_iters, mb * sizeof(int)));
+    MGB_CUDA(cudaMallocHost(&h_norm2, (8 + mb) * sizeof(double)));
+    MGB_CUDA(cudaMalloc(&d_loop, mb * sizeof(LoopState)));
+    MGB_CUDA(cudaMemsetAsync(d_loop, 0, mb * sizeof(LoopState), stream));
+    MGB_CUDA(cudaMallocHost(&h_loop, mb * sizeof(LoopState)));
+    if (batch > 0) {
+        MGB_CUDA(cudaMalloc(&d_active, mb * sizeof(int)));
+        MGB_CUDA(cudaMallocHost(&h_active, mb * sizeof(int)));
+        res0_b.assign(mb, 0.0); res_b.assign(mb, 0.0);
+        MGB_TRY(activate_all());
+    }
     MGB_CUDA(cudaStreamSynchronize(stream));
     if (P > 1) MGB_TRY(setup_p2p());
     return MGB200_OK;
@@ -354,7 +427,7 @@ int mgb200_solver::alloc_levels()
         g.L.row0 = g.mem_lo;
         if (!g.present) continue;
         g.elems = (size_t)g.L.pitch * (size_t)g.rows_mem();
-        const size_t bytes = g.elems * sizeof(double);
+        const size_t bytes = g.elems * sizeof(double) * (size_t)members();      // batched: the members back to back
         MGB_CUDA(cudaMalloc(&g.u[0], bytes));
         MGB_CUDA(cudaMalloc(&g.u[1], bytes));
         MGB_CUDA(cudaMalloc(&g.rhs, bytes));
@@ -661,11 +734,14 @@ int mgb200_solver::scatter_from_root(Level& c, double* arr)
 int mgb200_solver::build_towers()
 {
     if (maxlvl == 1) return MGB200_OK;
+    // (a batch: the towers of every member, one after another; member b of level l at + b * lv[l].elems)
+    auto mo = [&](int l, int b) { return (size_t)b * lv[l].elems; };
     if (opt.correct_towers) {
-        for (int l = 1; l < maxlvl; ++l) {
-            MGB_TRY(launch_restrict(lv[l].v1, lv[l].L, lv[l - 1].v1, lv[l - 1].L, lv[l - 1].n, stream));
-            MGB_TRY(launch_restrict(lv[l].v2, lv[l].L, lv[l - 1].v2, lv[l - 1].L, lv[l - 1].n, stream));
-        }
+        for (int b = 0; b < members(); ++b)
+            for (int l = 1; l < maxlvl; ++l) {
+                MGB_TRY(launch_restrict(lv[l].v1 + mo(l, b), lv[l].L, lv[l - 1].v1 + mo(l - 1, b), lv[l - 1].L, lv[l - 1].n, stream));
+                MGB_TRY(launch_restrict(lv[l].v2 + mo(l, b), lv[l].L, lv[l - 1].v2 + mo(l - 1, b), lv[l - 1].L, lv[l - 1].n, stream));
+            }
         return MGB200_OK;
     }
     // Reference-compatible: every level is restriction(dst, src, N/2) on flat zero-filled
@@ -677,8 +753,9 @@ int mgb200_solver::build_towers()
     // The flat mapping only reads rows 0..N/4+1 of the level-0 velocity.  A single GPU reads them
     // from its own level 0; a slab rank from the dense copy of those rows that set_fields left in
     // d_top (every rank builds every flat buffer redundantly and keeps the rows of its windows).
+    for (int b = 0; b < members(); ++b)
     for (int which = 0; which < 2; ++which) {
-        const double* src0 = P == 1 ? (which == 0 ? lv[0].v1 : lv[0].v2) : d_top[1 + which];
+        const double* src0 = P == 1 ? (which == 0 ? lv[0].v1 : lv[0].v2) + mo(0, b) : d_top[1 + which];
         const Layout L0 = P == 1 ? lv[0].L : natural_layout(N + 1);
         int cur = 0;
         for (int l = 1; l < maxlvl; ++l) {
@@ -686,7 +763,7 @@ int mgb200_solver::build_towers()
             if (l == 1) MGB_TRY(launch_tower_flat(d_flat[cur], src0, true, L0, N, stream));
             else MGB_TRY(launch_tower_flat(d_flat[cur], d_flat[1 - cur], false, L0, N, stream));
             if (lv[l].present) {
-                double* dst = which == 0 ? lv[l].v1 : lv[l].v2;
+                double* dst = (which == 0 ? lv[l].v1 : lv[l].v2) + mo(l, b);
                 MGB_TRY(launch_flat_to_level(dst, lv[l].L, d_flat[cur], lv[l].n, stream, lv[l].mem_lo, lv[l].mem_hi));
             }
             cur = 1 - cur;
@@ -715,6 +792,15 @@ int mgb200_solver::cycle_body(int l)
             // coarsest level: on-device loop {GS; residual; norm} (multigrid.cpp:55-65).  A level
             // entered from above starts from u = 0 (multigrid.cpp:77); the kernel zero-fills itself.
             const bool fresh = (l > 0 && rep == 0);
+            if (batch > 0) {
+                if (opt.coarse_exact)
+                    MGB_TRY(launch_coarse_lu_solve_batched(g.u[g.cur], g.rhs, g.v1, g.v2, d_coarse_lu, g.n, g.L, g.st, fresh, batch, (long)g.elems,
+                                                           (long)(coarse_lu_bytes(g.n) / sizeof(double)), d_active, stream));
+                else
+                    MGB_TRY(launch_coarse_solve_batched(g.u[g.cur], g.rhs, g.v1, g.v2, g.n, g.L, g.st, opt.arith, fresh, opt.coarse_maxit,
+                                                        opt.coarse_tol, d_coarse_iters, batch, (long)g.elems, d_active, stream));
+                continue;
+            }
             if (opt.coarse_exact) MGB_TRY(launch_coarse_lu_solve(g.u[g.cur], g.rhs, g.v1, g.v2, d_coarse_lu, g.n, g.L, g.st, fresh, stream));
             else MGB_TRY(launch_coarse_solve(g.u[g.cur], g.rhs, g.v1, g.v2, g.n, g.L, g.st, opt.arith, fresh,
                                              opt.coarse_maxit, opt.coarse_tol, d_coarse_iters, stream));
@@ -749,6 +835,7 @@ int mgb200_solver::cycle_body(int l)
                 a.Lc = c.L;
                 if (left == 0) { a.post = opt.restriction == MGB200_RESTRICT_FW ? POST_FW : POST_INJECT; a.coarse_rhs = c.rhs; }
                 fill_pass_window(a, g, c);
+                fill_pass_batch(a, g, c);
                 if (split) fill_pass_push(a, g, c, left == 0);
                 MGB_TRY(stream_pass(a, stream));
                 g.cur = 1 - g.cur;
@@ -783,6 +870,7 @@ int mgb200_solver::cycle_body(int l)
                 if (first) a.coarse_u = c.u[c.cur];
                 if (left == 0 && l == 0 && rep == opt.shape - 1) { a.post = POST_NORM2; a.partials = d_partials; }
                 fill_pass_window(a, g, c);
+                fill_pass_batch(a, g, c);
                 if (split) fill_pass_push(a, g, c, false);
                 MGB_TRY(stream_pass(a, stream));
                 g.cur = 1 - g.cur;
@@ -799,6 +887,14 @@ int mgb200_solver::cycle_body(int l)
 int mgb200_solver::residual_norm_level0()
 {
     Level& g = lv[0];
+    if (batch > 0) {
+        // a batched handle with one level: every member's norm (a frozen member's comes out as before: its u and rhs
+        // are unchanged), then the active members' sums
+        for (int b = 0; b < batch; ++b)
+            MGB_TRY(launch_residual(nullptr, g.u[g.cur] + (size_t)b * g.elems, g.rhs + (size_t)b * g.elems, g.v1 + (size_t)b * g.elems,
+                                    g.v2 + (size_t)b * g.elems, g.n, g.L, g.st, opt.arith, d_partials + (size_t)b * pstride, stream));
+        return launch_reduce_partials_batched(d_partials, residual_partials_count(g.n), pstride, d_norm2, d_active, batch, stream);
+    }
     MGB_TRY(launch_residual(nullptr, g.u[g.cur], g.rhs, g.v1, g.v2, g.n, g.L, g.st, opt.arith, d_partials, stream));
     MGB_TRY(launch_reduce_partials(d_partials, residual_partials_count(g.n), d_norm2, stream));
     return MGB200_OK;
@@ -811,6 +907,10 @@ int mgb200_solver::record_cycle()
     if (opt.plan == MGB200_PLAN_FUSED && maxlvl > 1) {
         // the level-0 up leg already produced the per-tile sums of squares (its LAST chunk did)
         const int last_k = opt.niter == 0 ? 0 : ((opt.niter - 1) % 3) + 1;
+        if (batch > 0) {
+            MGB_TRY(launch_reduce_partials_batched(d_partials, stream_pass_tiles(N, N + 1, last_k, batch), pstride, d_norm2, d_active, batch, stream));
+            return MGB200_OK;
+        }
         MGB_TRY(launch_reduce_partials(d_partials, stream_pass_tiles(N, lv[0].own_hi - lv[0].own_lo + 1, last_k), d_norm2, stream));
         MGB_TRY(allreduce_norm());
         mark("norm");
@@ -876,9 +976,11 @@ int mgb200_solver::build_loop_graph()
     e = cudaGraphConditionalHandleCreate(&h, graph, 0, 0);
     if (e != cudaSuccess) return bail("cudaGraphConditionalHandleCreate", e);
     cudaKernelNodeParams kp{};
-    double tol_ = tol; int maxc = opt.max_cycle;
+    double tol_ = tol; int maxc = opt.max_cycle, nmb = batch;
     void* args[] = {&h, &d_norm2, &d_loop, &tol_, &maxc};
+    void* bargs[] = {&h, &d_norm2, &d_loop, &d_active, &tol_, &maxc, &nmb};
     kp.func = (void*)k_loop_begin; kp.gridDim = dim3(1); kp.blockDim = dim3(1); kp.kernelParams = args;
+    if (batch > 0) { kp.func = (void*)k_loop_begin_batched; kp.blockDim = dim3(1024); kp.kernelParams = bargs; }
     cudaGraphNode_t n_begin, n_while;
     e = cudaGraphAddKernelNode(&n_begin, graph, nullptr, 0, &kp);
     if (e != cudaSuccess) return bail("cudaGraphAddKernelNode", e);
@@ -892,7 +994,8 @@ int mgb200_solver::build_loop_graph()
     e = cudaStreamBeginCaptureToGraph(stream, body, nullptr, nullptr, 0, cudaStreamCaptureModeThreadLocal);
     if (e != cudaSuccess) return bail("cudaStreamBeginCaptureToGraph", e);
     int rc = record_cycle();
-    if (rc == MGB200_OK) { k_loop_check<<<1, 1, 0, stream>>>(h, d_norm2, d_loop); rc = check_launch("k_loop_check"); }
+    if (rc == MGB200_OK && batch > 0) { k_loop_check_batched<<<1, 1024, 0, stream>>>(h, d_norm2, d_loop, d_active, batch); rc = check_launch("k_loop_check_batched"); }
+    else if (rc == MGB200_OK) { k_loop_check<<<1, 1, 0, stream>>>(h, d_norm2, d_loop); rc = check_launch("k_loop_check"); }
     cudaGraph_t captured = nullptr;
     e = cudaStreamEndCapture(stream, &captured);
     loop_kernels = launch_counter() - before;
@@ -922,6 +1025,19 @@ int mgb200_solver::form_rhs(double* res0_out, bool sync)
     if (!have_fields) return fail(MGB200_ERR_STATE, "form_rhs before set_fields");
     Level& g = lv[0];
     const long before = launch_counter();
+    if (batch > 0) {
+        MGB_TRY(activate_all());
+        MGB_TRY(launch_compute_rhs_batched(g.rhs, g.u[g.cur], g.v1, g.v2, g.n, g.L, g.st, opt.arith, d_partials, pstride, batch, (long)g.elems, stream));
+        MGB_TRY(launch_reduce_partials_batched(d_partials, compute_rhs_partials_count(g.n, g.n - 1, g.L), pstride, d_norm2, nullptr, batch, stream));
+        count(before);
+        have_rhs = true;
+        norm_is_res0 = true; res0_on_host = false;
+        if (!sync) return MGB200_OK;
+        MGB_TRY(read_norms(res0_out));
+        res0_b = res_b;
+        res0_on_host = true;
+        return MGB200_OK;
+    }
     if (P == 1) {
         MGB_TRY(launch_compute_rhs(g.rhs, g.u[g.cur], g.v1, g.v2, g.n, g.L, g.st, opt.arith, d_partials, stream));
         MGB_TRY(launch_reduce_partials(d_partials, compute_rhs_partials_count(g.n, g.n - 1, g.L), d_norm2, stream));
@@ -957,9 +1073,146 @@ bool report_solve(int cycles, int max_cycle, double res0, double res, double tol
 }
 }  // namespace mgb200
 
+void mgb200_solver::fill_pass_batch(StreamPassArgs& a, const Level& g, const Level& c) const
+{
+    if (batch == 0) return;
+    a.members = batch; a.mstride = (long)g.elems; a.cmstride = (long)c.elems; a.pstride = pstride; a.active = d_active;
+}
+
+int mgb200_solver::activate_all()
+{
+    k_fill_int<<<(batch + 255) / 256, 256, 0, stream>>>(d_active, batch, 1);
+    return check_launch("k_fill_int");
+}
+
+// every member's current norm -> res_b (and out[0..batch) if given)
+int mgb200_solver::read_norms(double* out)
+{
+    MGB_CUDA(cudaMemcpyAsync(h_norm2, d_norm2, (size_t)batch * sizeof(double), cudaMemcpyDeviceToHost, stream));
+    MGB_CUDA(cudaStreamSynchronize(stream));
+    for (int b = 0; b < batch; ++b) {
+        res_b[b] = std::sqrt(h_norm2[b]);                                         // gs.cpp:106
+        if (out) out[b] = res_b[b];
+    }
+    return MGB200_OK;
+}
+
+static void fill_info(mgb200_solve_info* info, const LoopState& ls, double tol)
+{
+    const int it = ls.iter;
+    std::memset(info, 0, sizeof(*info));
+    for (int k = 0; k <= it; ++k) info->hist[k] = ls.hist[k];
+    info->cycles = it; info->res0 = ls.res0; info->res = ls.hist[it]; info->converged = (info->res / info->res0 <= tol) ? 1 : 0;
+}
+
+// mg_outer for every member of a batch: each member runs its own loop (multigrid.cpp:108) and is frozen once its
+// condition fails; the cycles go on while any member runs.  infos: `batch` entries (may be null).
+int mgb200_solver::solve_batched(mgb200_solve_info* infos)
+{
+    if (!have_rhs) return fail(MGB200_ERR_STATE, "solve before form_rhs");
+    if (device_loop() && norm_is_res0 && !loop_exec) {
+        if (build_loop_graph() != MGB200_OK)
+            fprintf(stderr, "mgb200: device-side solve loop unavailable (%s); using the host loop\n", mgb200_last_error());
+    }
+    if (device_loop() && norm_is_res0 && loop_exec) {
+        MGB_CUDA(cudaGraphLaunch(loop_exec, stream));
+        MGB_CUDA(cudaMemcpyAsync(h_loop, d_loop, (size_t)batch * sizeof(LoopState), cudaMemcpyDeviceToHost, stream));
+        MGB_CUDA(cudaStreamSynchronize(stream));
+        norm_is_res0 = false; res0_on_host = true;
+        int trips = 0;
+        for (int b = 0; b < batch; ++b) {
+            const LoopState& ls = h_loop[b];
+            trips = std::max(trips, ls.iter);
+            res0_b[b] = ls.res0; res_b[b] = ls.hist[ls.iter];
+            if (infos) fill_info(&infos[b], ls, tol);
+            report_solve(ls.iter, opt.max_cycle, ls.res0, ls.hist[ls.iter], tol);
+        }
+        launches += 1 + (long)trips * loop_kernels;
+        return MGB200_OK;
+    }
+    if (!res0_on_host) {
+        if (!norm_is_res0) return fail(MGB200_ERR_STATE, "solve: initial residual norm unknown; call form_rhs first");
+        MGB_TRY(read_norms(nullptr));
+        res0_b = res_b;
+        res0_on_host = true;
+    }
+    std::vector<LoopState> ls((size_t)batch);
+    for (int b = 0; b < batch; ++b) {
+        ls[b].res0 = res0_b[b]; ls[b].iter = 0; ls[b].hist[0] = res0_b[b];
+        res_b[b] = res0_b[b];
+    }
+    std::vector<double> r(res0_b);
+    for (;;) {                                                                    // :108, per member
+        bool any = false;
+        for (int b = 0; b < batch; ++b) {
+            h_active[b] = (ls[b].iter < opt.max_cycle && r[b] / res0_b[b] > tol) ? 1 : 0;
+            any = any || h_active[b];
+        }
+        if (!any) break;
+        MGB_CUDA(cudaMemcpyAsync(d_active, h_active, (size_t)batch * sizeof(int), cudaMemcpyHostToDevice, stream));
+        MGB_TRY(run_cycle_async());                                               // :110-112
+        MGB_TRY(read_norms(nullptr));                                             // :113
+        for (int b = 0; b < batch; ++b)
+            if (h_active[b]) { r[b] = res_b[b]; ls[b].hist[++ls[b].iter] = r[b]; }
+    }
+    for (int b = 0; b < batch; ++b) {
+        if (infos) fill_info(&infos[b], ls[b], tol);
+        report_solve(ls[b].iter, opt.max_cycle, res0_b[b], r[b], tol);
+    }
+    return MGB200_OK;
+}
+
+// nsteps x { compute_rhs ; mg_outer } for every member; infos: nsteps x batch entries, step-major
+int mgb200_solver::timestep_batched(int nsteps, mgb200_solve_info* infos)
+{
+    if (nsteps <= 0) return MGB200_OK;
+    int k0 = 0;
+    if (device_loop() && !loop_exec) {
+        MGB_TRY(form_rhs(nullptr, false));
+        MGB_TRY(solve_batched(infos));
+        k0 = 1;
+    }
+    if (!(device_loop() && loop_exec)) {
+        for (int k = k0; k < nsteps; ++k) {
+            MGB_TRY(form_rhs(nullptr, false));
+            MGB_TRY(solve_batched(infos ? infos + (size_t)k * batch : nullptr));
+        }
+        return MGB200_OK;
+    }
+    const int todo = nsteps - k0;
+    if (todo <= 0) return MGB200_OK;
+    const long need = (long)todo * batch;
+    if (h_steps_cap < need) {
+        if (h_steps) cudaFreeHost(h_steps);
+        h_steps = nullptr; h_steps_cap = 0;
+        MGB_CUDA(cudaMallocHost(&h_steps, (size_t)need * sizeof(LoopState)));
+        h_steps_cap = (int)need;
+    }
+    for (int k = 0; k < todo; ++k) {
+        MGB_TRY(form_rhs(nullptr, false));
+        MGB_CUDA(cudaGraphLaunch(loop_exec, stream));
+        MGB_CUDA(cudaMemcpyAsync(&h_steps[(size_t)k * batch], d_loop, (size_t)batch * sizeof(LoopState), cudaMemcpyDeviceToHost, stream));
+    }
+    MGB_CUDA(cudaStreamSynchronize(stream));
+    norm_is_res0 = false; res0_on_host = true;
+    for (int k = 0; k < todo; ++k) {
+        int trips = 0;
+        for (int b = 0; b < batch; ++b) {
+            const LoopState& ls = h_steps[(size_t)k * batch + b];
+            trips = std::max(trips, ls.iter);
+            res0_b[b] = ls.res0; res_b[b] = ls.hist[ls.iter];
+            if (infos) fill_info(&infos[(size_t)(k0 + k) * batch + b], ls, tol);
+            report_solve(ls.iter, opt.max_cycle, ls.res0, ls.hist[ls.iter], tol);
+        }
+        launches += 1 + (long)trips * loop_kernels;
+    }
+    return MGB200_OK;
+}
+
 // mg_outer (multigrid.cpp:97-120)
 int mgb200_solver::solve(mgb200_solve_info* info)
 {
+    if (batch > 0) return solve_batched(info);
     if (!have_rhs) return fail(MGB200_ERR_STATE, "solve before form_rhs");
     if (device_loop() && norm_is_res0 && !loop_exec) {
         // every rank takes the same decision: the capture works everywhere or nowhere
@@ -1008,6 +1261,7 @@ int mgb200_solver::solve(mgb200_solve_info* info)
 // all steps back to back and the host synchronises once at the end.
 int mgb200_solver::timestep(int nsteps, mgb200_solve_info* infos)
 {
+    if (batch > 0) return timestep_batched(nsteps, infos);
     if (nsteps <= 0) return MGB200_OK;
     int k0 = 0;
     if (device_loop() && !loop_exec) {
@@ -1058,8 +1312,10 @@ int mgb200_solver::get_u_natural(double* dst_dev, long ld)
 {
     Level& g = lv[0];
     const long before = launch_counter();
-    // a slab rank fills its own rows only (the destination is a full-size array)
-    MGB_TRY(launch_convert(dst_dev, natural_layout(ld), g.u[g.cur], g.L, g.n, stream, g.own_lo, g.own_hi));
+    // a slab rank fills its own rows only (the destination is a full-size array); member b of a batch at + b (n+1) ld
+    for (int b = 0; b < members(); ++b)
+        MGB_TRY(launch_convert(dst_dev + (size_t)b * (g.n + 1) * ld, natural_layout(ld), g.u[g.cur] + (size_t)b * g.elems, g.L, g.n, stream,
+                               g.own_lo, g.own_hi));
     count(before);
     return MGB200_OK;
 }
@@ -1099,6 +1355,22 @@ int mgb200_create(mgb200_solver** out, long n, int maxlvl, double nu, double dt,
     *out = s;
     return MGB200_OK;
 }
+
+int mgb200_create_batched(mgb200_solver** out, long n, int maxlvl, int batch, double nu, double dt, double dx, double tol,
+                          const mgb200_options* opt)
+{
+    if (!out) return fail(MGB200_ERR_INVALID, "out == NULL");
+    *out = nullptr;
+    if (batch < 1) return fail(MGB200_ERR_INVALID, "create_batched: batch must be >= 1");
+    mgb200_solver* s = new mgb200_solver();
+    s->batch = batch;
+    int rc = s->init(n, maxlvl, nu, dt, dx, tol, opt);
+    if (rc != MGB200_OK) { delete s; return rc; }
+    *out = s;
+    return MGB200_OK;
+}
+
+int mgb200_batch_size(mgb200_solver* s) { return s ? s->members() : 0; }
 
 int mgb200_comm_unique_id(unsigned char id[128]) { return comm_unique_id(id); }
 
@@ -1176,8 +1448,10 @@ static int after_fields(mgb200_solver* s)
     if (s->opt.coarse_exact && (s->P == 1 || s->rank == 0)) {
         // the coarsest operator depends on the (new) velocities only: factor it once
         Level& c = s->lv[s->maxlvl - 1];
-        if (!s->d_coarse_lu) MGB_CUDA(cudaMalloc(&s->d_coarse_lu, coarse_lu_bytes(c.n)));
-        MGB_TRY(launch_coarse_lu_factor(s->d_coarse_lu, c.v1, c.v2, c.n, c.L, c.st, s->stream));
+        if (!s->d_coarse_lu) MGB_CUDA(cudaMalloc(&s->d_coarse_lu, coarse_lu_bytes(c.n) * s->members()));
+        for (int b = 0; b < s->members(); ++b)                  // (a batch: one factorisation per member)
+            MGB_TRY(launch_coarse_lu_factor(s->d_coarse_lu + b * (coarse_lu_bytes(c.n) / sizeof(double)), c.v1 + (size_t)b * c.elems,
+                                            c.v2 + (size_t)b * c.elems, c.n, c.L, c.st, s->stream));
     }
     if (s->P > 1) {                    // the tower inputs are no longer needed
         MGB_CUDA(cudaStreamSynchronize(s->stream));
@@ -1194,10 +1468,13 @@ int mgb200_set_fields_device(mgb200_solver* s, const double* u0, const double* v
     if (!s || !u0 || !v1 || !v2 || ld < s->N + 1) return fail(MGB200_ERR_INVALID, "set_fields_device: bad argument");
     Level& g = s->lv[0];
     const long before = launch_counter();
-    // (slab ranks take the rows of their window out of the full-size arrays)
-    MGB_TRY(launch_convert(g.u[g.cur], g.L, u0, natural_layout(ld), g.n, s->stream, g.mem_lo, g.mem_hi));
-    MGB_TRY(launch_convert(g.v1, g.L, v1, natural_layout(ld), g.n, s->stream, g.mem_lo, g.mem_hi));
-    MGB_TRY(launch_convert(g.v2, g.L, v2, natural_layout(ld), g.n, s->stream, g.mem_lo, g.mem_hi));
+    // (slab ranks take the rows of their window out of the full-size arrays; member b of a batch is at + b (n+1) ld)
+    for (int b = 0; b < s->members(); ++b) {
+        const size_t mo = (size_t)b * g.elems, io = (size_t)b * (g.n + 1) * ld;
+        MGB_TRY(launch_convert(g.u[g.cur] + mo, g.L, u0 + io, natural_layout(ld), g.n, s->stream, g.mem_lo, g.mem_hi));
+        MGB_TRY(launch_convert(g.v1 + mo, g.L, v1 + io, natural_layout(ld), g.n, s->stream, g.mem_lo, g.mem_hi));
+        MGB_TRY(launch_convert(g.v2 + mo, g.L, v2 + io, natural_layout(ld), g.n, s->stream, g.mem_lo, g.mem_hi));
+    }
     if (s->P > 1) {
         MGB_TRY(s->alloc_top());
         const long top = s->N / 4 + 1;
@@ -1240,6 +1517,24 @@ int mgb200_set_fields_host(mgb200_solver* s, const double* u0, const double* v1,
         return MGB200_OK;
     };
     if (s->P > 1) MGB_TRY(s->alloc_top());
+    if (s->batch > 0) {
+        // member b: host arrays at + b (n+1)^2, staged through its own idle twin and rhs
+        for (int b = 0; b < s->batch; ++b) {
+            const size_t mo = (size_t)b * g.elems, ho = (size_t)b * (n + 1) * (n + 1);
+            MGB_CUDA(cudaMemcpyAsync(stage_a + mo, u0 + ho, bytes, cudaMemcpyHostToDevice, s->stream));
+            MGB_TRY(launch_convert(g.u[g.cur] + mo, g.L, stage_a + mo, dense, n, s->stream));
+            MGB_CUDA(cudaMemcpyAsync(stage_b + mo, v1 + ho, bytes, cudaMemcpyHostToDevice, s->stream));
+            MGB_TRY(launch_convert(g.v1 + mo, g.L, stage_b + mo, dense, n, s->stream));
+            MGB_CUDA(cudaMemcpyAsync(stage_a + mo, v2 + ho, bytes, cudaMemcpyHostToDevice, s->stream));
+            MGB_TRY(launch_convert(g.v2 + mo, g.L, stage_a + mo, dense, n, s->stream));
+        }
+        MGB_CUDA(cudaMemsetAsync(stage_a, 0, g.elems * s->batch * sizeof(double), s->stream));
+        MGB_CUDA(cudaMemsetAsync(stage_b, 0, g.elems * s->batch * sizeof(double), s->stream));
+        MGB_TRY(after_fields(s));
+        s->count(before);
+        MGB_CUDA(cudaStreamSynchronize(s->stream));
+        return MGB200_OK;
+    }
     MGB_CUDA(cudaMemcpyAsync(stage_a, u0 + off, bytes, cudaMemcpyHostToDevice, s->stream));
     MGB_TRY(launch_convert(g.u[g.cur], g.L, stage_a, dense, n, s->stream, g.mem_lo, g.mem_hi));
     MGB_CUDA(cudaMemcpyAsync(stage_b, v1 + off, bytes, cudaMemcpyHostToDevice, s->stream));
@@ -1261,7 +1556,9 @@ int mgb200_set_fields_reference_ic(mgb200_solver* s, double vscale)
     if (!s) return fail(MGB200_ERR_INVALID, "solver == NULL");
     Level& g = s->lv[0];
     const long before = launch_counter();
-    MGB_TRY(launch_initial_conditions(g.u[g.cur], g.v1, g.v2, g.n, g.L, vscale, s->stream, g.mem_lo, g.mem_hi));
+    for (int b = 0; b < s->members(); ++b)      // (a batch: the same fields for every member)
+        MGB_TRY(launch_initial_conditions(g.u[g.cur] + (size_t)b * g.elems, g.v1 + (size_t)b * g.elems, g.v2 + (size_t)b * g.elems, g.n, g.L,
+                                          vscale, s->stream, g.mem_lo, g.mem_hi));
     if (s->P > 1) {
         MGB_TRY(s->alloc_top());
         MGB_TRY(launch_initial_conditions(s->d_top[0], s->d_top[1], s->d_top[2], g.n, natural_layout(g.n + 1), vscale, s->stream, 0, s->N / 4 + 1));
@@ -1280,6 +1577,11 @@ int mgb200_form_rhs(mgb200_solver* s, double* res0)
 int mgb200_cycle(mgb200_solver* s, double* res)
 {
     if (!s) return fail(MGB200_ERR_INVALID, "solver == NULL");
+    if (s->batch > 0) {                 // every member cycles
+        MGB_TRY(s->activate_all());
+        MGB_TRY(s->run_cycle_async());
+        return s->read_norms(res);
+    }
     MGB_TRY(s->run_cycle_async());
     return s->read_norm(res);
 }
@@ -1287,12 +1589,14 @@ int mgb200_cycle(mgb200_solver* s, double* res)
 int mgb200_cycle_async(mgb200_solver* s)
 {
     if (!s) return fail(MGB200_ERR_INVALID, "solver == NULL");
+    if (s->batch > 0) MGB_TRY(s->activate_all());
     return s->run_cycle_async();
 }
 
 int mgb200_last_norm(mgb200_solver* s, double* res)
 {
     if (!s) return fail(MGB200_ERR_INVALID, "solver == NULL");
+    if (s->batch > 0) return s->read_norms(res);
     return s->read_norm(res);
 }
 
@@ -1320,13 +1624,16 @@ int mgb200_get_u_host(mgb200_solver* s, double* u)
 {
     if (!s || !u) return fail(MGB200_ERR_INVALID, "get_u_host: bad argument");
     Level& g = s->lv[0];
-    double* stage = g.u[1 - g.cur];      // idle between passes
-    // dense staging of the OWNED rows (a slab rank fills only its rows of the full-size host array)
+    // dense staging of the OWNED rows (a slab rank fills only its rows of the full-size host array); member b of a
+    // batch goes to + b (n+1)^2, staged in its own idle twin
     const long before = launch_counter();
-    MGB_TRY(launch_convert(stage, natural_layout(g.n + 1, g.own_lo), g.u[g.cur], g.L, g.n, s->stream, g.own_lo, g.own_hi));
+    for (int b = 0; b < s->members(); ++b) {
+        double* stage = g.u[1 - g.cur] + (size_t)b * g.elems;      // idle between passes
+        MGB_TRY(launch_convert(stage, natural_layout(g.n + 1, g.own_lo), g.u[g.cur] + (size_t)b * g.elems, g.L, g.n, s->stream, g.own_lo, g.own_hi));
+        MGB_CUDA(cudaMemcpyAsync(u + (size_t)b * (g.n + 1) * (g.n + 1) + (size_t)g.own_lo * (g.n + 1), stage,
+                                 (size_t)(g.own_hi - g.own_lo + 1) * (g.n + 1) * sizeof(double), cudaMemcpyDeviceToHost, s->stream));
+    }
     s->count(before);
-    MGB_CUDA(cudaMemcpyAsync(u + (size_t)g.own_lo * (g.n + 1), stage, (size_t)(g.own_hi - g.own_lo + 1) * (g.n + 1) * sizeof(double),
-                             cudaMemcpyDeviceToHost, s->stream));
     MGB_CUDA(cudaStreamSynchronize(s->stream));
     // (the staging buffer is the next pass's output: every pass rewrites all owned rows of its output
     // and the exchange refreshes the halo rows, so nothing needs restoring)
@@ -1344,11 +1651,14 @@ int mgb200_get_level_host(mgb200_solver* s, int lvl, int which, double* out)
     const size_t bytes = (size_t)g.rows_mem() * (g.n + 1) * sizeof(double);
     out += (size_t)g.mem_lo * (g.n + 1);
     MGB_CUDA(cudaMalloc(&tmp, bytes));
-    int rc = launch_convert(tmp, natural_layout(g.n + 1, g.mem_lo), src, g.L, g.n, s->stream, g.mem_lo, g.mem_hi);
-    if (rc == MGB200_OK) {
-        cudaError_t e = cudaMemcpyAsync(out, tmp, bytes, cudaMemcpyDeviceToHost, s->stream);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(s->stream);
-        if (e != cudaSuccess) rc = fail(MGB200_ERR_CUDA, cudaGetErrorString(e));
+    int rc = MGB200_OK;
+    for (int b = 0; b < s->members() && rc == MGB200_OK; ++b) {       // member b of a batch: + b (n_l+1)^2
+        rc = launch_convert(tmp, natural_layout(g.n + 1, g.mem_lo), src + (size_t)b * g.elems, g.L, g.n, s->stream, g.mem_lo, g.mem_hi);
+        if (rc == MGB200_OK) {
+            cudaError_t e = cudaMemcpyAsync(out + (size_t)b * (g.n + 1) * (g.n + 1), tmp, bytes, cudaMemcpyDeviceToHost, s->stream);
+            if (e == cudaSuccess) e = cudaStreamSynchronize(s->stream);
+            if (e != cudaSuccess) rc = fail(MGB200_ERR_CUDA, cudaGetErrorString(e));
+        }
     }
     cudaFree(tmp);
     return rc;
@@ -1389,7 +1699,7 @@ double mgb200_cycle_bytes(mgb200_solver* s)
         total += per_node * m * mult * reps;
     }
     if (s->opt.plan == MGB200_PLAN_UNFUSED || s->maxlvl == 1) total += 32.0 * (double)(s->N + 1) * (double)(s->N + 1);
-    return total;
+    return total * s->members();        // a batch: every member's cycle
 }
 
 int mgb200_profile_level0(mgb200_solver* s, int reps, double* ms_a, double* bytes_a, double* ms_b, double* bytes_b)
@@ -1398,7 +1708,8 @@ int mgb200_profile_level0(mgb200_solver* s, int reps, double* ms_a, double* byte
     if (s->maxlvl < 2) return fail(MGB200_ERR_INVALID, "profile_level0: needs at least two levels");
     Level& g = s->lv[0];
     Level& c = s->lv[1];
-    const double m0 = (double)(g.own_hi - g.own_lo + 1) * (double)(g.n + 1);   // nodes this rank produces
+    const double m0 = (double)(g.own_hi - g.own_lo + 1) * (double)(g.n + 1) * s->members();   // nodes this rank produces (every member)
+    if (s->batch > 0) MGB_TRY(s->activate_all());
     cudaEvent_t e0, e1;
     MGB_CUDA(cudaEventCreate(&e0));
     MGB_CUDA(cudaEventCreate(&e1));
@@ -1418,6 +1729,7 @@ int mgb200_profile_level0(mgb200_solver* s, int reps, double* ms_a, double* byte
                 if (which == 0) { a.post = s->opt.restriction == MGB200_RESTRICT_FW ? POST_FW : POST_INJECT; a.coarse_rhs = c.rhs; }
                 else { a.coarse_u = c.u[c.cur]; a.post = POST_NORM2; a.partials = s->d_partials; }
                 s->fill_pass_window(a, g, c);
+                s->fill_pass_batch(a, g, c);
                 rc = stream_pass(a, s->stream);
                 g.cur = 1 - g.cur;
             } else if (which == 0) {

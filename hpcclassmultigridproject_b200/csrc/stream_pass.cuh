@@ -53,11 +53,21 @@ struct StreamPassArgs {
     long c_own_lo, c_own_hi;   // coarse rows this rank owns (for the coarse-rhs push)
     int* sync;
     int* raise_up; int* raise_dn;
+    // Batched pass (single GPU, whole levels): members >= 1 problems of this size in one launch (0: one problem, the
+    // plain kernel).  Member b of u_in / u_out / rhs / v1 / v2 starts b * mstride doubles after the first, of
+    // coarse_u / coarse_rhs b * cmstride after, its partial sums at partials + b * pstride.  active[b] == 0: member b
+    // is frozen, the pass leaves everything of it untouched.
+    int members;
+    long mstride, cmstride, pstride;
+    const int* active;
 };
 
 // number of tiles (= partial sums written by POST_NORM2) of a pass over level n with `iters`
-// fused iterations; iters < 1: the maximum over all iteration counts (buffer sizing)
-long stream_pass_tiles(long n, long nrows, int iters);
+// fused iterations; iters < 1: the maximum over all iteration counts (buffer sizing).  members: the pass's
+// StreamPassArgs::members (the count is per member)
+long stream_pass_tiles(long n, long nrows, int iters, int members = 0);
+// most members a batched pass takes (gridDim.y)
+constexpr int STREAM_PASS_MAX_MEMBERS = 65535;
 // one-time attribute setup
 int stream_pass_init();
 int stream_pass(const StreamPassArgs& a, cudaStream_t s);

@@ -54,6 +54,24 @@ SY_FN void sy_tma_prefetch(const Params& p, int which, int x, int z)
                  : "memory");
 }
 
+SY_FN void sy_tma_load_m(const Params& p, const Smem& sm, int which, unsigned soff, int x, int z, int m, int g)
+{
+    asm volatile(
+        "cp.async.bulk.tensor.4d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4, %5}], [%6];" ::"r"(
+            sm.base32 + soff),
+        "l"(&p.maps[which]), "r"(x), "r"(0), "r"(z), "r"(m), "r"(sm.base32 + sm.full_off + 8u * g)
+        : "memory");
+}
+
+SY_FN void sy_tma_prefetch_m(const Params& p, int which, int x, int z, int m)
+{
+    asm volatile("cp.async.bulk.prefetch.tensor.4d.L2.global.tile [%0, {%1, %2, %3, %4}];" ::"l"(&p.maps[which]), "r"(x), "r"(0), "r"(z),
+                 "r"(m)
+                 : "memory");
+}
+
+SY_FN int sy_member() { return (int)blockIdx.y; }
+
 __device__ __forceinline__ void mbar_wait(unsigned a, unsigned parity)
 {
     unsigned done;
@@ -191,6 +209,35 @@ __global__ void __launch_bounds__(THREADS, 1) k_syst_pass(const __grid_constant_
     }
 }
 
+// The batched flavour: grid (tiles, members), member blockIdx.y.  Single GPU, whole levels: none of the row-slab
+// machinery of k_syst_pass.  A frozen member's blocks leave before they touch anything, so its arrays and partial
+// sums keep what its last active pass left there.
+template <int ARITH, bool PRE, int POSTK>
+__global__ void __launch_bounds__(THREADS, 1) k_syst_pass_batched(const __grid_constant__ Params p)
+{
+    if (p.active[blockIdx.y] == 0) return;
+    extern __shared__ __align__(128) unsigned char smem_raw[];
+    __shared__ double scratch[32];
+    Smem sm;
+    carve(sm, smem_raw, p.SWK);
+    sm.base32 = smem_u32(smem_raw);
+    const Tile tl = make_tile(p, blockIdx.x, POSTK == POST_FW ? 1 : 0);
+    const Geo geo = make_geo(p);
+    const int warp = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0);
+    const int lane = threadIdx.x & 31;
+    if (threadIdx.x < NGROUP)
+        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(sm.base32 + sm.full_off + 8u * threadIdx.x) : "memory");
+    if (threadIdx.x < NPROG) *reinterpret_cast<volatile unsigned*>(smem_raw + sm.pb_off + 4u * threadIdx.x) = 0u;
+    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    sy_fence_async();
+    __syncthreads();
+    const double acc = run_warp<ARITH, PRE, POSTK, true>(p, tl, geo, sm, warp, lane);
+    if (POSTK == POST_NORM2) {
+        const double tot = block_sum(acc, scratch);
+        if (threadIdx.x == 0) p.partials[(long)blockIdx.y * p.pstride + blockIdx.x] = tot;
+    }
+}
+
 static int g_sms = 0;
 
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
@@ -200,15 +247,17 @@ static EncodeTiledFn g_encode = nullptr;
 
 // {run, parity, row} view of a split-layout field: dim0 = pairs of one run (stride 8 B, extent = the
 // run stride `odd`, slack included), dim1 = parity (stride odd*8), dim2 = rows (stride pitch*8).
-static int encode_field(TensorMapStorage* out, const double* base, long odd, long pitch, long rows, int box_x, int box_rows)
+// members > 0: a 4-D {run, parity, row, member} view of a batch (dim3 stride mstride*8), box one member deep.
+static int encode_field(TensorMapStorage* out, const double* base, long odd, long pitch, long rows, int box_x, int box_rows,
+                        int members = 0, long mstride = 0)
 {
     static_assert(sizeof(CUtensorMap) == sizeof(TensorMapStorage), "CUtensorMap size");
     CUtensorMap m;
-    const cuuint64_t dims[3] = {(cuuint64_t)odd, 2, (cuuint64_t)rows};
-    const cuuint64_t strides[2] = {(cuuint64_t)odd * 8, (cuuint64_t)pitch * 8};
-    const cuuint32_t box[3] = {(cuuint32_t)box_x, 2, (cuuint32_t)box_rows};
-    const cuuint32_t estr[3] = {1, 1, 1};
-    CUresult r = g_encode(&m, CU_TENSOR_MAP_DATA_TYPE_FLOAT64, 3, const_cast<double*>(base), dims, strides, box, estr,
+    const cuuint64_t dims[4] = {(cuuint64_t)odd, 2, (cuuint64_t)rows, (cuuint64_t)(members > 0 ? members : 1)};
+    const cuuint64_t strides[3] = {(cuuint64_t)odd * 8, (cuuint64_t)pitch * 8, (cuuint64_t)mstride * 8};
+    const cuuint32_t box[4] = {(cuuint32_t)box_x, 2, (cuuint32_t)box_rows, 1};
+    const cuuint32_t estr[4] = {1, 1, 1, 1};
+    CUresult r = g_encode(&m, CU_TENSOR_MAP_DATA_TYPE_FLOAT64, members > 0 ? 4 : 3, const_cast<double*>(base), dims, strides, box, estr,
                           CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                           CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (r != CUDA_SUCCESS) return fail(MGB200_ERR_CUDA, "cuTensorMapEncodeTiled failed with CUresult " + std::to_string((int)r));
@@ -216,17 +265,19 @@ static int encode_field(TensorMapStorage* out, const double* base, long odd, lon
     return MGB200_OK;
 }
 
-static Plan plan_for(long n, long nrows, int K)
+// members: StreamPassArgs::members (0 and 1 give the same plan)
+static Plan plan_for(long n, long nrows, int K, int members = 0)
 {
-    static std::map<std::tuple<long, long, int>, Plan> cache;
+    static std::map<std::tuple<long, long, int, int>, Plan> cache;
     static std::mutex mu;
     std::lock_guard<std::mutex> lock(mu);
-    auto key = std::make_tuple(n, nrows, K);
+    const int mb = members > 1 ? members : 1;
+    auto key = std::make_tuple(n, nrows, K, mb);
     auto it = cache.find(key);
     if (it == cache.end()) {
         int force = 0;
         if (const char* e = getenv("MGB200_SWK")) force = atoi(e);       // tuning aid: pin the strip width
-        it = cache.emplace(key, make_plan(n, nrows, K, g_sms > 0 ? g_sms : 148, force)).first;
+        it = cache.emplace(key, make_plan(n, nrows, K, g_sms > 0 ? g_sms : 148, force, mb)).first;
     }
     return it->second;
 }
@@ -245,6 +296,20 @@ static PassKernel pass_kernel(int arith, bool pre, int post)
     // full weighting: down leg only, no prolongation flavour
     if (post == POST_FW) return arith == MGB200_ARITH_EXACT ? k_syst_pass<MGB200_ARITH_EXACT, false, POST_FW> : k_syst_pass<MGB200_ARITH_FAST, false, POST_FW>;
     return arith == MGB200_ARITH_EXACT ? pass_kernel_of<MGB200_ARITH_EXACT>(pre, post) : pass_kernel_of<MGB200_ARITH_FAST>(pre, post);
+}
+
+template <int ARITH>
+static PassKernel batched_kernel_of(bool pre, int post)
+{
+    if (post == POST_FW) return k_syst_pass_batched<ARITH, false, POST_FW>;
+    if (pre) return post == POST_NORM2 ? k_syst_pass_batched<ARITH, true, POST_NORM2> : post == POST_INJECT ? k_syst_pass_batched<ARITH, true, POST_INJECT>
+                                                                                                           : k_syst_pass_batched<ARITH, true, POST_NONE>;
+    return post == POST_NORM2 ? k_syst_pass_batched<ARITH, false, POST_NORM2> : post == POST_INJECT ? k_syst_pass_batched<ARITH, false, POST_INJECT>
+                                                                                                     : k_syst_pass_batched<ARITH, false, POST_NONE>;
+}
+static PassKernel batched_kernel(int arith, bool pre, int post)
+{
+    return arith == MGB200_ARITH_EXACT ? batched_kernel_of<MGB200_ARITH_EXACT>(pre, post) : batched_kernel_of<MGB200_ARITH_FAST>(pre, post);
 }
 
 }  // namespace sy
@@ -267,6 +332,12 @@ int stream_pass_init()
                 MGB_CUDA(cudaFuncSetAttribute(pass_kernel(arith, pre != 0, post), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_BYTES));
     for (int arith = 0; arith < 2; ++arith)
         MGB_CUDA(cudaFuncSetAttribute(pass_kernel(arith, false, POST_FW), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_BYTES));
+    for (int arith = 0; arith < 2; ++arith) {
+        for (int pre = 0; pre < 2; ++pre)
+            for (int post = 0; post < 3; ++post)
+                MGB_CUDA(cudaFuncSetAttribute(batched_kernel(arith, pre != 0, post), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_BYTES));
+        MGB_CUDA(cudaFuncSetAttribute(batched_kernel(arith, false, POST_FW), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_BYTES));
+    }
     if (!g_encode) {
         void* fn = nullptr;
         cudaDriverEntryPointQueryResult qres;
@@ -278,15 +349,15 @@ int stream_pass_init()
     return MGB200_OK;
 }
 
-long stream_pass_tiles(long n, long nrows, int iters)
+long stream_pass_tiles(long n, long nrows, int iters, int members)
 {
     if (iters >= 1) {
-        const Plan pl = plan_for(n, nrows, iters > KMAX ? KMAX : iters);
+        const Plan pl = plan_for(n, nrows, iters > KMAX ? KMAX : iters, members);
         return (long)pl.nstrips * pl.nbands;
     }
     long m = 0;
     for (int K = 1; K <= KMAX; ++K) {
-        const Plan pl = plan_for(n, nrows, K);
+        const Plan pl = plan_for(n, nrows, K, members);
         m = std::max(m, (long)pl.nstrips * pl.nbands);
     }
     return m;
@@ -300,7 +371,11 @@ static int build_params(const StreamPassArgs& a, Params& p, unsigned& grid_out, 
     MGB_TRY(stream_pass_init());
     const bool whole = a.rows_mem == 0;
     const long own_lo = whole ? 0 : a.own_lo, own_hi = whole ? a.n : a.own_hi;
-    const Plan pl = plan_for(a.n, own_hi - own_lo + 1, a.iters);
+    if (a.members < 0 || a.members > STREAM_PASS_MAX_MEMBERS) return fail(MGB200_ERR_INVALID, "stream_pass: members must be 0..65535");
+    const bool batch = a.members > 0;
+    if (batch && (!whole || !a.active || a.mstride <= 0 || (a.coarse_u && a.cmstride <= 0) || a.sync))
+        return fail(MGB200_ERR_INVALID, "stream_pass: a batched pass needs whole levels, member strides and the active flags");
+    const Plan pl = plan_for(a.n, own_hi - own_lo + 1, a.iters, a.members);
     p = Params{};
     p.n = a.n; p.nhalf = a.n / 2;
     p.own_lo = own_lo; p.own_hi = own_hi;
@@ -319,12 +394,14 @@ static int build_params(const StreamPassArgs& a, Params& p, unsigned& grid_out, 
     p.st = a.st;
     p.u_in = a.u_in; p.rhs = a.rhs; p.v1 = a.v1; p.v2 = a.v2; p.cu = a.coarse_u;
     // the u map of a zero-input pass is never dereferenced (its boxes lie out of bounds): any valid field will do
-    MGB_TRY(encode_field(&p.maps[FIELD_U], a.u_in ? a.u_in : a.rhs, a.L.odd, a.L.pitch, p.rows_mem, pl.SWK, GROUP));
-    MGB_TRY(encode_field(&p.maps[FIELD_F], a.rhs, a.L.odd, a.L.pitch, p.rows_mem, pl.SWK, GROUP));
-    MGB_TRY(encode_field(&p.maps[FIELD_V1], a.v1, a.L.odd, a.L.pitch, p.rows_mem, pl.SWK, GROUP));
-    MGB_TRY(encode_field(&p.maps[FIELD_V2], a.v2, a.L.odd, a.L.pitch, p.rows_mem, pl.SWK, GROUP));
-    if (a.coarse_u) MGB_TRY(encode_field(&p.maps[FIELD_C], a.coarse_u, a.Lc.odd, a.Lc.pitch, p.crows_mem, p.CW, CROWS));
+    const int mb = a.members;
+    MGB_TRY(encode_field(&p.maps[FIELD_U], a.u_in ? a.u_in : a.rhs, a.L.odd, a.L.pitch, p.rows_mem, pl.SWK, GROUP, mb, a.mstride));
+    MGB_TRY(encode_field(&p.maps[FIELD_F], a.rhs, a.L.odd, a.L.pitch, p.rows_mem, pl.SWK, GROUP, mb, a.mstride));
+    MGB_TRY(encode_field(&p.maps[FIELD_V1], a.v1, a.L.odd, a.L.pitch, p.rows_mem, pl.SWK, GROUP, mb, a.mstride));
+    MGB_TRY(encode_field(&p.maps[FIELD_V2], a.v2, a.L.odd, a.L.pitch, p.rows_mem, pl.SWK, GROUP, mb, a.mstride));
+    if (a.coarse_u) MGB_TRY(encode_field(&p.maps[FIELD_C], a.coarse_u, a.Lc.odd, a.Lc.pitch, p.crows_mem, p.CW, CROWS, mb, a.cmstride));
     p.u_out = a.u_out; p.crhs = a.coarse_rhs; p.partials = a.partials;
+    if (batch) { p.mstride = a.mstride; p.cmstride = a.cmstride; p.pstride = a.pstride; p.active = a.active; }
     p.peer_u_up = a.peer_u_up; p.peer_u_dn = a.peer_u_dn; p.peer_c_up = a.peer_c_up; p.peer_c_dn = a.peer_c_dn;
     p.push_rows = a.push_rows; p.c_own_lo = a.c_own_lo; p.c_own_hi = a.c_own_hi;
     p.sync = a.sync; p.raise_up = a.raise_up; p.raise_dn = a.raise_dn;
@@ -333,6 +410,7 @@ static int build_params(const StreamPassArgs& a, Params& p, unsigned& grid_out, 
     if (p.post == POST_NORM2 && !p.partials) return fail(MGB200_ERR_INVALID, "stream_pass: POST_NORM2 without partials");
     grid_out = (unsigned)(pl.nstrips * pl.nbands);
     smem_out = smem_bytes(pl.SWK);
+    if (batch && p.post == POST_NORM2 && a.pstride < (long)grid_out) return fail(MGB200_ERR_INVALID, "stream_pass: partials stride below the tile count");
     return MGB200_OK;
 }
 
@@ -342,7 +420,7 @@ int stream_pass(const StreamPassArgs& a, cudaStream_t s)
     // only on the argument record: a solver issues the same few dozen passes every cycle, so blocks
     // are built once and looked up by the raw bytes of the arguments (per device: tensor maps hold
     // device addresses, which are unique across the devices of a process).
-    struct Entry { Params p; unsigned grid; size_t smem; };
+    struct Entry { Params p; unsigned grid; size_t smem; int members; };
     static std::map<std::string, Entry> cache;
     static std::mutex mu;
     Entry e;
@@ -357,15 +435,21 @@ int stream_pass(const StreamPassArgs& a, cudaStream_t s)
         key.peer_u_up = a.peer_u_up; key.peer_u_dn = a.peer_u_dn; key.peer_c_up = a.peer_c_up; key.peer_c_dn = a.peer_c_dn;
         key.push_rows = a.push_rows; key.c_own_lo = a.c_own_lo; key.c_own_hi = a.c_own_hi; key.sync = a.sync;
         key.raise_up = a.raise_up; key.raise_dn = a.raise_dn;
+        key.members = a.members; key.mstride = a.mstride; key.cmstride = a.cmstride; key.pstride = a.pstride; key.active = a.active;
         std::string k(reinterpret_cast<const char*>(&key), sizeof(key));
         auto it = cache.find(k);
         if (it == cache.end()) {
             Entry fresh;
             MGB_TRY(build_params(a, fresh.p, fresh.grid, fresh.smem));
+            fresh.members = a.members;
             if (cache.size() > 4096) cache.clear();     // many short-lived solvers: do not grow without bound
             it = cache.emplace(std::move(k), fresh).first;
         }
         e = it->second;                                 // copied under the lock: the map may be cleared by another thread
+    }
+    if (e.members > 0) {
+        batched_kernel(a.arith, e.p.pre != 0, e.p.post)<<<dim3(e.grid, (unsigned)e.members), THREADS, e.smem, s>>>(e.p);
+        return check_launch("k_syst_pass_batched");
     }
     pass_kernel(a.arith, e.p.pre != 0, e.p.post)<<<e.grid, THREADS, e.smem, s>>>(e.p);
     return check_launch("k_syst_pass");

@@ -104,6 +104,10 @@ struct Params {
     double* peer_u_up; double* peer_u_dn; double* peer_c_up; double* peer_c_dn;
     long push_rows, c_own_lo, c_own_hi;
     int* sync; int* raise_up; int* raise_dn;
+    // batched passes (k_syst_pass_batched): member b of every fine / coarse array starts b * mstride / b * cmstride
+    // doubles after the first, its partial sums at b * pstride; a member whose active[b] is 0 is not touched
+    long mstride, cmstride, pstride;
+    const int* active;
 };
 
 struct Tile {
@@ -169,6 +173,19 @@ SY_FN void sy_full_expect(const Smem& sm, int g, unsigned bytes);
 // is (pair x, parity 0, memory row z) of the field; out-of-bounds elements arrive as zeros
 SY_FN void sy_tma_load(const Params& p, const Smem& sm, int which, unsigned soff, int x, int z, int g);
 SY_FN void sy_tma_prefetch(const Params& p, int which, int x, int z);   // same box, into L2 only
+// batched passes: the maps are 4-D {pair, parity, row, member}; the same box (one member deep) of member m, zeros
+// outside that member's rows
+SY_FN void sy_tma_load_m(const Params& p, const Smem& sm, int which, unsigned soff, int x, int z, int m, int g);
+SY_FN void sy_tma_prefetch_m(const Params& p, int which, int x, int z, int m);
+SY_FN int sy_member();                                   // batched passes: the member of this block
+// first element of this block's member in an array whose members lie `stride` doubles apart (0 unless BATCH; the
+// batched primitives are only named in batched code, so a host model without them still builds the others)
+template <bool BATCH>
+SY_FN long member_off(long stride)
+{
+    if constexpr (BATCH) return (long)sy_member() * stride;
+    else return 0L;
+}
 SY_FN void sy_full_wait(const Smem& sm, int g, unsigned parity);
 // progress counters: steps completed by a stage warp.  Publish = store-release by one lane after
 // sy_syncwarp (orders the whole warp's earlier shared-memory writes); peek = load-acquire of the
@@ -395,9 +412,10 @@ SY_FN void pre_loop(const Params& p, const Tile& tl, const Geo& geo, const Smem&
 // Coarse right-hand side node pair (cr, kg), (cr, kg+1) of a lane whose vector starts at global pair kg (even: the
 // strips start at even pairs): kg -> E run at kg/2, kg+1 -> O run; only the owned interior columns (rmask0), and
 // the same values into the slab neighbours' halo rows of the coarse rhs.
+template <bool BATCH>
 SY_FN void store_coarse(const Params& p, const Stage& st, long kg, long cr, double r0, double r1)
 {
-    double* crow = p.crhs + (cr - p.crow0) * p.cpitch + (kg >> 1);
+    double* crow = p.crhs + member_off<BATCH>(p.cmstride) + (cr - p.crow0) * p.cpitch + (kg >> 1);
     if (st.rmask0 & 1u) crow[0] = r0;
     if (st.rmask0 & 2u) crow[p.codd] = r1;
     if (p.peer_c_up && cr < p.c_own_lo + p.push_rows) {
@@ -429,6 +447,7 @@ SY_FN double fw_row(double a, double b, double c, double w)
 // from this role -- once the other EPI warp has published row q as well (lane 0 reads that warp's last node).  The
 // horizontal sums of the lane's two coarse columns J = kg, kg+1 (fine columns 2J-1, 2J, 2J+1 = O[J-1], E[J], O[J])
 // are kept in registers: an even row waits in fw.e, an odd row 2I+1 completes coarse row I and becomes fw.o.
+template <bool BATCH>
 SY_FN void fw_restrict_row(const Params& p, const Tile& tl, const Geo& geo, const Smem& sm, const Stage& st, FwSums& fw,
                            const int k, const int q, const bool live)
 {
@@ -441,7 +460,7 @@ SY_FN void fw_restrict_row(const Params& p, const Tile& tl, const Geo& geo, cons
     const D2 h{fw_row(ol, e.x, o.x, w), fw_row(o.x, e.y, o.y, w)};
     if ((q & 1) == 0) { fw.e = h; return; }
     if (q - 1 >= st.elo && q - 1 <= st.ehi)
-        store_coarse(p, st, (long)tl.k0 + st.kk, (long)(q >> 1), __dadd_rn(__dadd_rn(fw.o.x, fw.e.x), h.x),
+        store_coarse<BATCH>(p, st, (long)tl.k0 + st.kk, (long)(q >> 1), __dadd_rn(__dadd_rn(fw.o.x, fw.e.x), h.x),
                      __dadd_rn(__dadd_rn(fw.o.y, fw.e.y), h.y));
     fw.o = h;
 }
@@ -460,7 +479,7 @@ SY_FN void fw_restrict_row(const Params& p, const Tile& tl, const Geo& geo, cons
 //   FULL    steady state of a strip that touches neither side of the domain: the update is active and every lane
 //           stores (the strip's outermost pairs are halo: what is computed there is never used), so the step
 //           carries no mask, no range test and no predicated load
-template <int ARITH, bool LAST, bool NORM1, bool RESID, int EPI, bool FULL>
+template <int ARITH, bool LAST, bool NORM1, bool RESID, int EPI, bool FULL, bool BATCH>
 SY_FN void stage_step(const Params& p, const Tile& tl, const Geo& geo, const Smem& sm, Stage& st, const int k, const int PAR,
                       const bool CHECKED, FwSums* fw)
 {
@@ -543,7 +562,7 @@ SY_FN void stage_step(const Params& p, const Tile& tl, const Geo& geo, const Sme
             sy_sts2(sm, fw_off(tl, geo, st, row) + po, D2{r0, r1});
         }
         publish(sm, st, k);
-        fw_restrict_row(p, tl, geo, sm, st, *fw, k, row - 1, live);
+        fw_restrict_row<BATCH>(p, tl, geo, sm, st, *fw, k, row - 1, live);
     } else {
         publish(sm, st, k);                              // nothing written: only the rows' release is signalled
         if (work && row >= st.elo && row <= st.ehi && (EPI == POST_NORM2 || (row & 1) == 0)) {
@@ -551,7 +570,7 @@ SY_FN void stage_step(const Params& p, const Tile& tl, const Geo& geo, const Sme
             const double r1 = Arith<ARITH>::residual(f.y, own.y, up.y, n1, dn.y, n2, c1, p.st);
             if (EPI == POST_INJECT) {
                 // gs.cpp:283: coarse node (row/2, kg) for fine even column 2kg
-                store_coarse(p, st, (long)tl.k0 + st.kk, row >> 1, r0, r1);
+                store_coarse<BATCH>(p, st, (long)tl.k0 + st.kk, row >> 1, r0, r1);
             } else {
                 if (rm & 1u) st.acc += r0 * r0;
                 if (rm & 2u) st.acc += r1 * r1;
@@ -562,7 +581,7 @@ SY_FN void stage_step(const Params& p, const Tile& tl, const Geo& geo, const Sme
     advance_row(geo, st);
 }
 
-template <int ARITH, bool LAST, bool NORM1, bool RESID, int EPI, int XR = 0>
+template <int ARITH, bool LAST, bool NORM1, bool RESID, int EPI, int XR = 0, bool BATCH = false>
 SY_FN void stage_loop(const Params& p, const Tile& tl, const Geo& geo, const Smem& sm, Stage& st)
 {
     const int klast = last_step(p, tl, XR) - tl.R0;
@@ -579,20 +598,20 @@ SY_FN void stage_loop(const Params& p, const Tile& tl, const Geo& geo, const Sme
     // a strip that touches neither side of the domain runs the mask-free step (every lane must be live)
     const bool full = !RESID && tl.k0 >= 1 && (long)tl.k0 + p.SWK <= p.nhalf && (p.SWK & 63) == 0;
     for (; k <= klast && (k < kchk || par != 0); ++k, par ^= 1)
-        stage_step<ARITH, LAST, NORM1, RESID, EPI, false>(p, tl, geo, sm, st, k, par, true, &fw);
+        stage_step<ARITH, LAST, NORM1, RESID, EPI, false, BATCH>(p, tl, geo, sm, st, k, par, true, &fw);
     if (full) {
         for (; k + 1 <= kmain; k += 2) {
-            stage_step<ARITH, LAST, NORM1, RESID, EPI, true>(p, tl, geo, sm, st, k, 0, false, &fw);
-            stage_step<ARITH, LAST, NORM1, RESID, EPI, true>(p, tl, geo, sm, st, k + 1, 1, false, &fw);
+            stage_step<ARITH, LAST, NORM1, RESID, EPI, true, BATCH>(p, tl, geo, sm, st, k, 0, false, &fw);
+            stage_step<ARITH, LAST, NORM1, RESID, EPI, true, BATCH>(p, tl, geo, sm, st, k + 1, 1, false, &fw);
         }
     } else {
         for (; k + 1 <= kmain; k += 2) {
-            stage_step<ARITH, LAST, NORM1, RESID, EPI, false>(p, tl, geo, sm, st, k, 0, false, &fw);
-            stage_step<ARITH, LAST, NORM1, RESID, EPI, false>(p, tl, geo, sm, st, k + 1, 1, false, &fw);
+            stage_step<ARITH, LAST, NORM1, RESID, EPI, false, BATCH>(p, tl, geo, sm, st, k, 0, false, &fw);
+            stage_step<ARITH, LAST, NORM1, RESID, EPI, false, BATCH>(p, tl, geo, sm, st, k + 1, 1, false, &fw);
         }
     }
     for (; k <= klast; ++k, par ^= 1)
-        stage_step<ARITH, LAST, NORM1, RESID, EPI, false>(p, tl, geo, sm, st, k, par, true, &fw);
+        stage_step<ARITH, LAST, NORM1, RESID, EPI, false, BATCH>(p, tl, geo, sm, st, k, par, true, &fw);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -600,6 +619,7 @@ SY_FN void stage_loop(const Params& p, const Tile& tl, const Geo& geo, const Sme
 // coarse rows its prolongation needs, all completing on the slot's full barrier; then start the HBM
 // fetch of the group after next, whose shared-memory request will hit L2.  Whole (converged) warp,
 // warp-uniform operands; one elected lane issues.
+template <bool BATCH>
 SY_FN void issue_group_loads(const Params& p, const Tile& tl, const Geo& geo, const Smem& sm, int g)
 {
     if (!sy_elect()) return;
@@ -609,6 +629,23 @@ SY_FN void issue_group_loads(const Params& p, const Tile& tl, const Geo& geo, co
     sy_full_expect(sm, gs, 4u * fine + (p.pre ? geo.cgrpb : 0u));
     const unsigned so = (unsigned)gs * fine;
     // a zero iterate is produced by a box that lies entirely below the last memory row
+    if constexpr (BATCH) {                                           // the same boxes of member sy_member()
+        const int m = sy_member();
+        sy_tma_load_m(p, sm, FIELD_U, so, tl.k0, p.u_is_zero ? (int)p.rows_mem + 64 : z, m, gs);
+        sy_tma_load_m(p, sm, FIELD_F, so + geo.ringb, tl.k0, z, m, gs);
+        sy_tma_load_m(p, sm, FIELD_V1, so + 2u * geo.ringb, tl.k0, z, m, gs);
+        sy_tma_load_m(p, sm, FIELD_V2, so + 3u * geo.ringb, tl.k0, z, m, gs);
+        if (p.pre)
+            sy_tma_load_m(p, sm, FIELD_C, 4u * geo.ringb + (unsigned)gs * geo.cgrpb, tl.k0 / 2, (z >> 1), m, gs);
+        const int zp = z + 2 * GROUP;
+        if (g + 2 >= NGROUP && zp <= tl.R1) {
+            if (!p.u_is_zero) sy_tma_prefetch_m(p, FIELD_U, tl.k0, zp, m);
+            sy_tma_prefetch_m(p, FIELD_F, tl.k0, zp, m);
+            sy_tma_prefetch_m(p, FIELD_V1, tl.k0, zp, m);
+            sy_tma_prefetch_m(p, FIELD_V2, tl.k0, zp, m);
+        }
+        return;
+    }
     sy_tma_load(p, sm, FIELD_U, so, tl.k0, p.u_is_zero ? (int)p.rows_mem + 64 : z, gs);
     sy_tma_load(p, sm, FIELD_F, so + geo.ringb, tl.k0, z, gs);
     sy_tma_load(p, sm, FIELD_V1, so + 2u * geo.ringb, tl.k0, z, gs);
@@ -636,7 +673,7 @@ SY_FN void issue_group_loads(const Params& p, const Tile& tl, const Geo& geo, co
 // rows: once it has published its step on row rl it needs no row <= rl any more (what it still uses of row rl+1 it
 // carries in registers), so group g (first row G), which replaces rows G-RING .. G-RING+GROUP-1 (ring group g - NGROUP),
 // is requested once row G-RING+GROUP-1 is published and the store warp has counted that group.
-template <int XR = 0>
+template <int XR = 0, bool BATCH = false>
 SY_FN void store_loop(const Params& p, const Tile& tl, const Geo& geo, const Smem& sm)
 {
     const int klast = last_step(p, tl, XR) - tl.R0;
@@ -648,7 +685,7 @@ SY_FN void store_loop(const Params& p, const Tile& tl, const Geo& geo, const Sme
     const unsigned nO8 = (unsigned)((eO - tl.kb) * 8);
     int rs = tl.R0 - off_s;                                          // the last stage's row in step 0
     const long pitch = p.pitch;
-    double* gstE = p.u_out + ((long)rs - p.row0) * pitch + tl.kb;    // destinations of the row's two runs
+    double* gstE = p.u_out + member_off<BATCH>(p.mstride) + ((long)rs - p.row0) * pitch + tl.kb;    // destinations of the row's two runs
     double* gstO = gstE + p.odd;
     unsigned a = (unsigned)((((rs - tl.R0) % RING) + RING) % RING) * geo.rowb + (unsigned)HK * 8u;
     const unsigned awrap = geo.ringb + (unsigned)HK * 8u;
@@ -699,12 +736,12 @@ SY_FN void store_loop(const Params& p, const Tile& tl, const Geo& geo, const Sme
     if (sy_elect()) { sy_store_commit(); sy_store_wait_all(); sy_prog_publish(sm, 2 * PAIR_STORE, groups + 64u); }
 }
 
-template <int XR = 0>
+template <int XR = 0, bool BATCH = false>
 SY_FN void producer_loop(const Params& p, const Tile& tl, const Geo& geo, const Smem& sm)
 {
     const int ng = num_groups(tl);
     int gnext = 0;
-    for (; gnext < ng && gnext < NGROUP; ++gnext) issue_group_loads(p, tl, geo, sm, gnext);   // fresh slots
+    for (; gnext < ng && gnext < NGROUP; ++gnext) issue_group_loads<BATCH>(p, tl, geo, sm, gnext);   // fresh slots
     const int klast = last_step(p, tl, XR) - tl.R0;
     const int pair_s = 2 * p.K - 1, off_s = off_stage(p, pair_s);
     const bool epi = p.post != POST_NONE;
@@ -717,13 +754,14 @@ SY_FN void producer_loop(const Params& p, const Tile& tl, const Geo& geo, const 
         // ring group gnext - NGROUP must have left shared memory: the store warp has counted gnext - NGROUP + 1 groups
         prog_wait(sm, PAIR_STORE, (unsigned)(gnext - NGROUP + 1), 0u, sy_prog_peek(sm, PAIR_STORE));
         if (sy_elect()) sy_fence_async();                            // the stages' stores into the slots -> the engine's writes
-        issue_group_loads(p, tl, geo, sm, gnext);
+        issue_group_loads<BATCH>(p, tl, geo, sm, gnext);
         ++gnext;
     }
 }
 
-// the work of one warp on one tile; returns the thread's share of the POST_NORM2 sum
-template <int ARITH, bool PRE, int POSTK>
+// the work of one warp on one tile; returns the thread's share of the POST_NORM2 sum.  BATCH: the tile belongs to
+// member sy_member() of a batch, whose fields the 4-D tensor maps address
+template <int ARITH, bool PRE, int POSTK, bool BATCH = false>
 SY_FN double run_warp(const Params& p, const Tile& tl, const Geo& geo, const Smem& sm, int warp, int lane)
 {
     constexpr int XR = POSTK == POST_FW ? 2 : 0;       // extra steps of every role (last_step)
@@ -733,14 +771,14 @@ SY_FN double run_warp(const Params& p, const Tile& tl, const Geo& geo, const Sme
 #ifdef SY_HOST_MODEL
         if (lane != 0) return 0.0;
 #endif
-        producer_loop<XR>(p, tl, geo, sm);
+        producer_loop<XR, BATCH>(p, tl, geo, sm);
         return 0.0;
     }
     if (warp == STORE_WARP) {
 #ifdef SY_HOST_MODEL
         if (lane != 0) return 0.0;
 #endif
-        store_loop<XR>(p, tl, geo, sm);
+        store_loop<XR, BATCH>(p, tl, geo, sm);
         return 0.0;
     }
     const int pair = warp / NSTW, h = warp % NSTW;
@@ -755,15 +793,15 @@ SY_FN double run_warp(const Params& p, const Tile& tl, const Geo& geo, const Sme
     if (pair == PAIR_EPI) {
         if (POSTK == POST_NONE) return 0.0;
         Stage st = init_role(p, tl, geo, PAIR_EPI, last, 2 * p.K, off_epi(p), h, lane);
-        stage_loop<ARITH, false, false, true, POSTK, XR>(p, tl, geo, sm, st);
+        stage_loop<ARITH, false, false, true, POSTK, XR, BATCH>(p, tl, geo, sm, st);
         return st.acc;
     }
     if (pair > last) return 0.0;
     Stage st = init_role(p, tl, geo, pair, pair == 0 ? (PRE ? PAIR_PRE : -1) : pair - 1, pair, off_stage(p, pair), h, lane);
     // (the last stage differs from the others only where it sums or stores its own residual)
-    if (pair == last && POSTK == POST_NORM2) stage_loop<ARITH, true, true, false, POST_NONE>(p, tl, geo, sm, st);
-    else if (pair == last && POSTK == POST_FW) stage_loop<ARITH, true, false, false, POST_FW, XR>(p, tl, geo, sm, st);
-    else stage_loop<ARITH, false, false, false, POST_NONE, XR>(p, tl, geo, sm, st);
+    if (pair == last && POSTK == POST_NORM2) stage_loop<ARITH, true, true, false, POST_NONE, 0, BATCH>(p, tl, geo, sm, st);
+    else if (pair == last && POSTK == POST_FW) stage_loop<ARITH, true, false, false, POST_FW, XR, BATCH>(p, tl, geo, sm, st);
+    else stage_loop<ARITH, false, false, false, POST_NONE, XR, BATCH>(p, tl, geo, sm, st);
     return st.acc;
 }
 
@@ -771,11 +809,12 @@ SY_FN double run_warp(const Params& p, const Tile& tl, const Geo& geo, const Sme
 // Tile planner.  Cost model (relative): a tile takes (rows + fill) steps, a step costs
 // c0 + SWK (latency + work proportional to the strip width); tiles run one per SM in waves of
 // `sms`.  Search strip width (SWK a multiple of 16: TMA boxes land 128-byte aligned) and band
-// count for the cheapest plan.
+// count for the cheapest plan.  A batched pass runs the same tiles for each of `members` members,
+// so its waves count members x tiles (members = 1: the plan of a single problem).
 struct Plan { int WK, SWK, nstrips, nbands; long RBAND; };
 
 // n: level size (columns); nrows: rows this launch produces (n+1 on a single GPU, the slab otherwise)
-inline Plan make_plan(long n, long nrows, int K, int sms, int force_swk = 0)
+inline Plan make_plan(long n, long nrows, int K, int sms, int force_swk = 0, int members = 1)
 {
     const long npairs = n / 2 + 1;
     Plan best{};
@@ -788,7 +827,7 @@ inline Plan make_plan(long n, long nrows, int K, int sms, int force_swk = 0)
             const long RB = (nrows + nb - 1) / nb;
             if (nb > 1 && RB < 8) break;
             const int nbands = (int)((nrows + RB - 1) / RB);
-            const long tiles = (long)nstrips * nbands;
+            const long tiles = (long)nstrips * nbands * members;
             const long waves = (tiles + sms - 1) / sms;
             const double steps = (double)RB + 2.0 * (2 * K + 1) + 4.0 * K + 2.0 * GROUP;
             const double per_step = 96.0 + SWK;

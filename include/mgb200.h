@@ -164,6 +164,27 @@ int mgb200_create(mgb200_solver **out, long n, int maxlvl, double nu, double dt,
 int mgb200_destroy(mgb200_solver *s);
 
 /* ------------------------------------------------------------------------------------------
+ * Batched handle: `batch` >= 1 independent problems ("members") of one grid size advanced by the same
+ * kernel launches (no reference counterpart).  All members share n, maxlvl, nu, dt, dx, tol and the
+ * options; each has its own u0, v1, v2, coarse towers and cycle count.  In solve / timestep every
+ * member runs mg_outer's loop on its own and is frozen once its condition fails (its fields stay as a
+ * handle of that problem alone would leave them); the cycles go on while any member runs.  A member's
+ * u on every level, cycle counts and converged flags equal those of a single-problem handle bit for
+ * bit; its norms may differ from one in the last bits for batch >= 2 (the per-tile partial sums follow
+ * the batch's tiling).  Fused plan with niter >= 1 only (MGB200_ERR_INVALID otherwise), at most 65535
+ * members.  The calls of the single-problem handle take or return `batch` consecutive items:
+ *   set_fields_host / set_fields_device / get_u_*: member b at + b*(n+1)*ld doubles (ld = n+1 on the host);
+ *   get_level_host: batch dense (n_l+1)^2 arrays;  set_fields_reference_ic: the same fields for every member;
+ *   form_rhs, cycle, last_norm: batch norms;  cycle / cycle_async: every member cycles;
+ *   solve: batch infos;  timestep: nsteps x batch infos, step-major (infos[k*batch + b]).
+ * cycle_bytes and profile_level0 count every member.
+ * ------------------------------------------------------------------------------------------ */
+int mgb200_create_batched(mgb200_solver **out, long n, int maxlvl, int batch, double nu, double dt,
+                          double dx, double tol, const mgb200_options *opt);
+/* members of the handle: `batch` for a batched handle, 1 for every other */
+int mgb200_batch_size(mgb200_solver *s);
+
+/* ------------------------------------------------------------------------------------------
  * Row-slab sharding over the GPUs of one node, one process per GPU (no reference counterpart: the
  * reference is single-GPU; SURVEY.md section 8e).  Rank 0 calls mgb200_comm_unique_id and the host
  * program broadcasts the 128 bytes (bench.py uses torch.distributed); every rank then calls
