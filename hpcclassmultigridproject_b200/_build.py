@@ -49,15 +49,5 @@ def build(force: bool = False, verbose: bool = False) -> str:
     return LIB
 
 
-def build_variant(define: str, out_name: str) -> str:
-    """the library with a compile-time variant of the streaming pass (tuning experiments; MGB200_LIB selects it)"""
-    nvcc = shutil.which("nvcc") or "/usr/local/cuda/bin/nvcc"
-    out = os.path.join(HERE, out_name)
-    env = dict(os.environ)
-    env.pop("CC", None); env.pop("CXX", None)
-    subprocess.run([nvcc, *NVCC_FLAGS, "-D" + define, "-o", out, *sources()], check=True, env=env)
-    return out
-
-
 if __name__ == "__main__":
     print(build(force=True, verbose=True))

@@ -7,7 +7,7 @@ import math
 import os
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-LIB_PATH = os.environ.get("MGB200_LIB") or os.path.join(HERE, "libmgb200.so")   # MGB200_LIB: a tuning variant of the library
+LIB_PATH = os.environ.get("MGB200_LIB") or os.path.join(HERE, "libmgb200.so")   # MGB200_LIB: load the library from another path
 
 ARITH_FAST, ARITH_EXACT = 0, 1
 PLAN_FUSED, PLAN_UNFUSED = 0, 1

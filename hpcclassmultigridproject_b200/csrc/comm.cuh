@@ -38,17 +38,13 @@ int comm_allgather_bytes(Comm* c, const void* send, void* recv, size_t bytes, cu
 //                                                      4: norm contributions, 5: norm result from rank 0)
 //   [8..15]  arrivals this rank has consumed so far
 //   [16]     CTA arrival counter of the running launch
+//   [19]     set when a wait gave up (a peer never arrived within ~2 s: it died or left the sequence); the host
+//            checks it after synchronising and reports MGB200_ERR_STATE
 // Graph-replayable: every counter lives in device memory, nothing changes in the kernel arguments
 // between cycles.  Never run two ranks of one communicator on the same GPU (the waiter would spin
 // against a kernel that cannot be scheduled).
-//   [6..7]   arrivals of the halo pushes FUSED into the streaming passes (slot 6: from rank-1, 7: from rank+1):
-//            every pass on a sharded level raises them once when it ends; they are compared with
-//   [17]     the number of such passes this rank has completed
-//   [18]     CTA arrival counter of the running pass
-//   [19]     set when a wait gave up (a peer never arrived within ~2 s: it died or left the sequence); the host
-//            checks it after synchronising and reports MGB200_ERR_STATE
 constexpr int SYNC_FROM_UP = 0, SYNC_FROM_DOWN = 1, SYNC_GATHER = 2, SYNC_SCATTER = 3, SYNC_NORM_UP = 4, SYNC_NORM_DOWN = 5,
-              SYNC_PASS_UP = 6, SYNC_PASS_DOWN = 7, SYNC_PASSES_DONE = 17, SYNC_PASS_CTAS = 18, SYNC_ABORT = 19, SYNC_INTS = 32;
+              SYNC_ABORT = 19, SYNC_INTS = 32;
 // spin budget of a device-side wait for a peer, in clock64 ticks (~2 s)
 constexpr long long SYNC_SPIN_BUDGET = 4000000000LL;
 struct PeerSeg { const double* src; double* dst; long count; };      // count doubles, multiple of 2, 16-byte aligned

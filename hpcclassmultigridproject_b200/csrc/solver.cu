@@ -104,6 +104,31 @@ static Slab child_slab_of(long n_fine, int P, int rank)
     return w;
 }
 
+// The sharding rule: the row window of `rank` at level `lvl` of an n-point hierarchy of maxlvl levels over P ranks.
+// A level is cut into slabs while it is not the coarsest, its slabs keep shard_min_rows and 2 SLAB_HALO rows each,
+// and every finer level is cut too.  The other levels live whole on rank 0; the first of them also as the slab under
+// each other rank's fine slab.  Pure arithmetic: mgb200_slab_plan gives it without a GPU.
+struct Window { bool sharded, present; Slab rows; };
+static Window slab_window(long n, int maxlvl, int P, int rank, long shard_min_rows, int lvl)
+{
+    Window w{};
+    int last = -1;                     // the coarsest level cut so far
+    for (int l = 0; l <= lvl; ++l) {
+        const long nl = n >> l;
+        w = Window{false, true, Slab{0, nl, 0, nl}};
+        if (P == 1) continue;
+        if (l < maxlvl - 1 && nl / P >= shard_min_rows && nl / P >= 2 * SLAB_HALO && last == l - 1) {
+            w.sharded = true;
+            w.rows = slab_of(nl, P, rank);
+            last = l;
+        } else if (rank != 0) {
+            if (l == last + 1 && l > 0) w.rows = child_slab_of(n >> (l - 1), P, rank);
+            else w.present = false;
+        }
+    }
+    return w;
+}
+
 // mg_outer's loop state (multigrid.cpp:100-116) when the loop itself runs on the device
 struct LoopState {
     double res0, tol;
@@ -280,8 +305,6 @@ struct mgb200_solver {
     int  alloc_levels();
     int  alloc_top();
     void fill_pass_window(StreamPassArgs& a, const Level& g, const Level& c) const;
-    bool fused_push = false;           // halo rows stored into the neighbours by the passes themselves (peer memory only)
-    void fill_pass_push(StreamPassArgs& a, const Level& g, const Level& c, bool coarse_rhs_too) const;
     int  exchange_halo(Level& g, double* a, Level* g2 = nullptr, double* a2 = nullptr);
     int  gather_to_root(Level& c, double* arr);
     int  scatter_from_root(Level& c, double* arr);
@@ -406,23 +429,10 @@ int mgb200_solver::alloc_levels()
         g.n = N >> l;
         g.L = split_layout(g.n);
         g.st = make_stencil(dt, nu, dx * (double)(1L << l));    // dx2 = 2*dx per level (multigrid.cpp:49)
-        g.own_lo = 0; g.own_hi = g.n; g.mem_lo = 0; g.mem_hi = g.n; g.sharded = false; g.present = true;
-        if (P > 1) {
-            const bool can = l < maxlvl - 1 && (g.n / P) >= shard_min_rows && (g.n / P) >= 2 * SLAB_HALO && last_sharded == l - 1;
-            if (can) {
-                const Slab w = slab_of(g.n, P, rank);
-                g.own_lo = w.own_lo; g.own_hi = w.own_hi; g.mem_lo = w.mem_lo; g.mem_hi = w.mem_hi;
-                g.sharded = true;
-                last_sharded = l;
-            } else if (rank != 0) {
-                if (l == last_sharded + 1 && l > 0) {           // slab of the first agglomerated level
-                    const Slab w = child_slab_of(lv[l - 1].n, P, rank);
-                    g.own_lo = w.own_lo; g.own_hi = w.own_hi; g.mem_lo = w.mem_lo; g.mem_hi = w.mem_hi;
-                } else {
-                    g.present = false;
-                }
-            }
-        }
+        const Window w = slab_window(N, maxlvl, P, rank, shard_min_rows, l);
+        g.own_lo = w.rows.own_lo; g.own_hi = w.rows.own_hi; g.mem_lo = w.rows.mem_lo; g.mem_hi = w.rows.mem_hi;
+        g.sharded = w.sharded; g.present = w.present;
+        if (g.sharded) last_sharded = l;
         if (P > 1 && l == 0 && !g.sharded) return fail(MGB200_ERR_INVALID, "level 0 is too small to be cut over the ranks");
         g.L.row0 = g.mem_lo;
         if (!g.present) continue;
@@ -457,30 +467,6 @@ void mgb200_solver::fill_pass_window(StreamPassArgs& a, const Level& g, const Le
     a.own_lo = g.own_lo; a.own_hi = g.own_hi;
     a.row0 = g.mem_lo; a.rows_mem = g.rows_mem();
     a.crow0 = c.mem_lo; a.crows_mem = c.rows_mem();
-}
-
-// Row slabs over peer memory: the pass itself stores the rows its neighbours need (its first / last SLAB_HALO rows of
-// the new iterate and, if the child level is sharded too, of the coarse right-hand side) into their halo rows and
-// raises their arrival counters when it ends; the neighbours' next pass waits for that in its edge tiles only.
-// One raise per pass and neighbour: every rank runs the same sequence of passes on the sharded levels, so "the
-// neighbour has finished as many passes as I have" is the whole protocol (comm.cuh, slots 6 / 7 / 17).
-void mgb200_solver::fill_pass_push(StreamPassArgs& a, const Level& g, const Level& c, bool coarse_rhs_too) const
-{
-    if (!(P > 1 && p2p && fused_push && g.sharded)) return;
-    const int l = (int)(&g - lv.data());
-    const int twin = a.u_out == g.u[0] ? 0 : 1;
-    a.sync = d_sync; a.push_rows = SLAB_HALO;
-    a.c_own_lo = c.own_lo; a.c_own_hi = c.own_hi;
-    for (int d = 0; d < 2; ++d) {
-        const int nb = d == 0 ? rank - 1 : rank + 1;
-        if (nb < 0 || nb >= P) continue;
-        const Slab w = slab_of(g.n, P, nb);
-        double* pu = peers[nb].lv[l].u[twin] - w.mem_lo * g.L.pitch;        // addressed by global row
-        double* pc = nullptr;
-        if (coarse_rhs_too && c.sharded) pc = peers[nb].lv[l + 1].rhs - slab_of(c.n, P, nb).mem_lo * c.L.pitch;
-        if (d == 0) { a.peer_u_up = pu; a.peer_c_up = pc; a.raise_up = peers[nb].sync + SYNC_PASS_DOWN; }   // we are its lower neighbour
-        else { a.peer_u_dn = pu; a.peer_c_dn = pc; a.raise_dn = peers[nb].sync + SYNC_PASS_UP; }
-    }
 }
 
 // Map the other ranks' arrays into this process (CUDA IPC over NVLink peer access): the slab
@@ -553,10 +539,6 @@ int mgb200_solver::setup_p2p()
     MGB_CUDA(cudaMemcpyAsync(&flag, d_flat_scratch(), sizeof(double), cudaMemcpyDeviceToHost, stream));
     MGB_CUDA(cudaStreamSynchronize(stream));
     p2p = flag > P - 0.5;
-    // MGB200_FUSED_PUSH=1: the passes store their boundary rows into the neighbours themselves (fill_pass_push).
-    // Opt-in: measured at 2 and 8 GPUs it saves the eight exchange launches of a cycle but not the wait for the
-    // neighbour, which is what an exchange costs (profiles/README.md), and the replayed graph is 2-3 % slower with it.
-    { const char* f = getenv("MGB200_FUSED_PUSH"); fused_push = p2p && f && atoi(f) != 0; }
     if (!p2p) {
         for (void* m : ipc_mapped) cudaIpcCloseMemHandle(m);
         ipc_mapped.clear();
@@ -836,20 +818,17 @@ int mgb200_solver::cycle_body(int l)
                 if (left == 0) { a.post = opt.restriction == MGB200_RESTRICT_FW ? POST_FW : POST_INJECT; a.coarse_rhs = c.rhs; }
                 fill_pass_window(a, g, c);
                 fill_pass_batch(a, g, c);
-                if (split) fill_pass_push(a, g, c, left == 0);
                 MGB_TRY(stream_pass(a, stream));
                 g.cur = 1 - g.cur;
                 first = false;
-                if (split && left > 0 && !a.sync) MGB_TRY(exchange_halo(g, g.u[g.cur]));
+                if (split && left > 0) MGB_TRY(exchange_halo(g, g.u[g.cur]));
             } while (left > 0);
             mark("L" + std::to_string(l) + "dn");
             if (split) {
                 // the new iterate's halo rows (read by the up leg) and the coarse right-hand side: halo rows to the
-                // slab neighbours (stored by the pass itself over peer memory, else by an exchange), or everything
-                // to rank 0 if the child is agglomerated
-                const bool pushed = p2p && fused_push;
-                if (c.sharded) { if (!pushed) MGB_TRY(exchange_halo(g, g.u[g.cur], &c, c.rhs)); }
-                else { if (!pushed) MGB_TRY(exchange_halo(g, g.u[g.cur])); MGB_TRY(gather_to_root(c, c.rhs)); }
+                // slab neighbours, or everything to rank 0 if the child is agglomerated
+                if (c.sharded) MGB_TRY(exchange_halo(g, g.u[g.cur], &c, c.rhs));
+                else { MGB_TRY(exchange_halo(g, g.u[g.cur])); MGB_TRY(gather_to_root(c, c.rhs)); }
             }
             mark("L" + std::to_string(l) + "x");
             if (runs_level(l + 1)) MGB_TRY(cycle_body(l + 1));
@@ -871,12 +850,11 @@ int mgb200_solver::cycle_body(int l)
                 if (left == 0 && l == 0 && rep == opt.shape - 1) { a.post = POST_NORM2; a.partials = d_partials; }
                 fill_pass_window(a, g, c);
                 fill_pass_batch(a, g, c);
-                if (split) fill_pass_push(a, g, c, false);
                 MGB_TRY(stream_pass(a, stream));
                 g.cur = 1 - g.cur;
                 first = false;
                 mark("L" + std::to_string(l) + "up");
-                if (split && !a.sync) { MGB_TRY(exchange_halo(g, g.u[g.cur])); mark("L" + std::to_string(l) + "x"); }
+                if (split) { MGB_TRY(exchange_halo(g, g.u[g.cur])); mark("L" + std::to_string(l) + "x"); }
             } while (left > 0);
         }
     }
@@ -1397,31 +1375,11 @@ int mgb200_create_sharded(mgb200_solver** out, long n, int maxlvl, double nu, do
 
 int mgb200_slab_plan(long n, int maxlvl, int nranks, int rank, long shard_min_rows, int lvl, long out[6])
 {
-    // pure arithmetic (no GPU): the row window of `rank` at level `lvl` under the sharding rule of
-    // alloc_levels.  out = {sharded, present, own_lo, own_hi, mem_lo, mem_hi}
+    // the window alloc_levels gives `rank` at level `lvl`.  out = {sharded, present, own_lo, own_hi, mem_lo, mem_hi}
     if (!out || lvl < 0 || lvl >= maxlvl || nranks < 1 || rank < 0 || rank >= nranks) return fail(MGB200_ERR_INVALID, "slab_plan: bad argument");
     if (shard_min_rows <= 0) shard_min_rows = 256;
-    int last = -1;
-    for (int l = 0; l <= lvl; ++l) {
-        const long nl = n >> l;
-        long w[6] = {0, 1, 0, nl, 0, nl};
-        if (nranks > 1) {
-            const bool can = l < maxlvl - 1 && (nl / nranks) >= shard_min_rows && (nl / nranks) >= 2 * SLAB_HALO && last == l - 1;
-            if (can) {
-                const Slab q = slab_of(nl, nranks, rank);
-                w[0] = 1; w[2] = q.own_lo; w[3] = q.own_hi; w[4] = q.mem_lo; w[5] = q.mem_hi;
-                last = l;
-            } else if (rank != 0) {
-                if (l == last + 1 && l > 0) {
-                    const Slab q = child_slab_of(n >> (l - 1), nranks, rank);
-                    w[2] = q.own_lo; w[3] = q.own_hi; w[4] = q.mem_lo; w[5] = q.mem_hi;
-                } else {
-                    w[1] = 0;
-                }
-            }
-        }
-        if (l == lvl) std::memcpy(out, w, sizeof(w));
-    }
+    const Window w = slab_window(n, maxlvl, nranks, rank, shard_min_rows, lvl);
+    out[0] = w.sharded; out[1] = w.present; out[2] = w.rows.own_lo; out[3] = w.rows.own_hi; out[4] = w.rows.mem_lo; out[5] = w.rows.mem_hi;
     return MGB200_OK;
 }
 

@@ -40,23 +40,10 @@ struct StreamPassArgs {
     long own_lo, own_hi;    // rows to produce
     long row0, rows_mem;    // fine arrays hold global rows row0 .. row0+rows_mem-1
     long crow0, crows_mem;  // same for the coarse arrays
-    // Halo push fused into the pass (row slabs over NVLink peer memory; all null / 0 otherwise).  The pass stores
-    // the first / last `push_rows` rows it produces (and the matching rows of the coarse rhs of a POST_INJECT / POST_FW
-    // pass whose child level is sharded too) straight into the slab neighbours' halo rows, raises their arrival
-    // counters when it ends and, at its start, lets only the tiles that stage halo rows wait for the
-    // neighbours' previous pass.  peer_*: the neighbours' copies of u_out / coarse_rhs, addressed like ours
-    // (pointer to THEIR memory row of global row 0, i.e. base - row0 * pitch); sync: this rank's counter block
-    // (comm.cuh); raise_*: the neighbours' arrival counters.
-    double* peer_u_up; double* peer_u_dn;
-    double* peer_c_up; double* peer_c_dn;
-    long push_rows;         // halo depth (rows), fine and coarse
-    long c_own_lo, c_own_hi;   // coarse rows this rank owns (for the coarse-rhs push)
-    int* sync;
-    int* raise_up; int* raise_dn;
-    // Batched pass (single GPU, whole levels): members >= 1 problems of this size in one launch (0: one problem, the
-    // plain kernel).  Member b of u_in / u_out / rhs / v1 / v2 starts b * mstride doubles after the first, of
-    // coarse_u / coarse_rhs b * cmstride after, its partial sums at partials + b * pstride.  active[b] == 0: member b
-    // is frozen, the pass leaves everything of it untouched.
+    // Batched pass (single GPU, whole levels): members >= 1 problems of this size in one launch (0: one problem).
+    // Member b of u_in / u_out / rhs / v1 / v2 starts b * mstride doubles after the first, of coarse_u / coarse_rhs
+    // b * cmstride after, its partial sums at partials + b * pstride.  active[b] == 0: member b is frozen, the pass
+    // leaves everything of it untouched.
     int members;
     long mstride, cmstride, pstride;
     const int* active;

@@ -11,7 +11,6 @@
 #include <string>
 #include <tuple>
 
-#include "comm.cuh"
 #include "syst_pass_body.cuh"
 
 namespace mgb200 {
@@ -100,22 +99,7 @@ SY_FN Prog2 sy_prog_peek(const Smem& sm, int stage)
     return v;
 }
 
-SY_FN void sy_backoff(int ns)
-{
-    if (ns > 0) __nanosleep((unsigned)ns);
-}
-
-SY_FN void sy_wait_neighbour(int* sync, int slot)
-{
-    const int want = *reinterpret_cast<volatile int*>(sync + SYNC_PASSES_DONE);
-    int seen;
-    const long long t0 = clock64();
-    do {
-        asm volatile("ld.acquire.sys.global.s32 %0, [%1];" : "=r"(seen) : "l"(sync + slot) : "memory");
-        if (seen - want < 0 && clock64() - t0 > SYNC_SPIN_BUDGET) { sync[SYNC_ABORT] = 1; break; }   // the peer is gone
-    } while (seen - want < 0);
-    asm volatile("fence.proxy.async;" ::: "memory");   // the rows that arrived are read by the TMA engine
-}
+SY_FN void sy_backoff(int) {}
 
 SY_FN void sy_bulk_store(const Smem& sm, double* gdst, unsigned soff, unsigned bytes)
 {
@@ -159,10 +143,13 @@ SY_FN double sy_side(const Smem& sm, const D2& mid, unsigned off, int dir, bool 
 
 // One kernel image per pass flavour (PRE: prolongation folded into stage 0; POSTK: epilogue kind
 // folded into the last stage): each image holds only the loops it runs, and the hot loops of all
-// roles together stay well inside the SM's instruction cache.
-template <int ARITH, bool PRE, int POSTK>
+// roles together stay well inside the SM's instruction cache.  BATCH: grid (tiles, members), the block
+// works on member blockIdx.y; a frozen member's blocks leave before they touch anything, so its arrays and
+// partial sums keep what its last active pass left there.
+template <int ARITH, bool PRE, int POSTK, bool BATCH>
 __global__ void __launch_bounds__(THREADS, 1) k_syst_pass(const __grid_constant__ Params p)
 {
+    if (BATCH && p.active[blockIdx.y] == 0) return;
     extern __shared__ __align__(128) unsigned char smem_raw[];
     __shared__ double scratch[32];
     Smem sm;
@@ -179,62 +166,11 @@ __global__ void __launch_bounds__(THREADS, 1) k_syst_pass(const __grid_constant_
     if (threadIdx.x < NPROG) *reinterpret_cast<volatile unsigned*>(smem_raw + sm.pb_off + 4u * threadIdx.x) = 0u;
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     sy_fence_async();
-    // row slabs with the halo push fused into the passes: a tile that stages rows (fine, or coarse for the
-    // prolongation) near a slab edge waits until the neighbour on that side has finished its previous pass
-    if (p.sync && threadIdx.x == 0) {
-        if (p.raise_up && tl.R0 - 8 < (int)p.own_lo) sy_wait_neighbour(p.sync, SYNC_PASS_UP);
-        if (p.raise_dn && tl.R1 + 8 > (int)p.own_hi) sy_wait_neighbour(p.sync, SYNC_PASS_DOWN);
-    }
     __syncthreads();
-    const double acc = run_warp<ARITH, PRE, POSTK>(p, tl, geo, sm, warp, lane);
-    if (p.sync) {
-        // the stores of the tiles near a slab edge into the neighbours' memory (only those tiles pay for the
-        // system-scope fence), then (last CTA) the neighbours' arrival counters
-        const bool pushed = (p.raise_up && tl.rb0 < (int)(p.own_lo + 2 * p.push_rows + 2)) || (p.raise_dn && tl.rb1 > (int)(p.own_hi - 2 * p.push_rows - 2));
-        if (pushed) __threadfence_system();
-        __syncthreads();
-        if (threadIdx.x == 0) {
-            unsigned* ctas = reinterpret_cast<unsigned*>(p.sync + SYNC_PASS_CTAS);
-            if (atomicInc(ctas, gridDim.x - 1) == gridDim.x - 1) {      // wraps to 0 for the next pass
-                __threadfence_system();
-                if (p.raise_up) atomicAdd_system(p.raise_up, 1);
-                if (p.raise_dn) atomicAdd_system(p.raise_dn, 1);
-                p.sync[SYNC_PASSES_DONE] += 1;
-            }
-        }
-    }
+    const double acc = run_warp<ARITH, PRE, POSTK, BATCH>(p, tl, geo, sm, warp, lane);
     if (POSTK == POST_NORM2) {
         const double tot = block_sum(acc, scratch);
-        if (threadIdx.x == 0) p.partials[blockIdx.x] = tot;
-    }
-}
-
-// The batched flavour: grid (tiles, members), member blockIdx.y.  Single GPU, whole levels: none of the row-slab
-// machinery of k_syst_pass.  A frozen member's blocks leave before they touch anything, so its arrays and partial
-// sums keep what its last active pass left there.
-template <int ARITH, bool PRE, int POSTK>
-__global__ void __launch_bounds__(THREADS, 1) k_syst_pass_batched(const __grid_constant__ Params p)
-{
-    if (p.active[blockIdx.y] == 0) return;
-    extern __shared__ __align__(128) unsigned char smem_raw[];
-    __shared__ double scratch[32];
-    Smem sm;
-    carve(sm, smem_raw, p.SWK);
-    sm.base32 = smem_u32(smem_raw);
-    const Tile tl = make_tile(p, blockIdx.x, POSTK == POST_FW ? 1 : 0);
-    const Geo geo = make_geo(p);
-    const int warp = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0);
-    const int lane = threadIdx.x & 31;
-    if (threadIdx.x < NGROUP)
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(sm.base32 + sm.full_off + 8u * threadIdx.x) : "memory");
-    if (threadIdx.x < NPROG) *reinterpret_cast<volatile unsigned*>(smem_raw + sm.pb_off + 4u * threadIdx.x) = 0u;
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    sy_fence_async();
-    __syncthreads();
-    const double acc = run_warp<ARITH, PRE, POSTK, true>(p, tl, geo, sm, warp, lane);
-    if (POSTK == POST_NORM2) {
-        const double tot = block_sum(acc, scratch);
-        if (threadIdx.x == 0) p.partials[(long)blockIdx.y * p.pstride + blockIdx.x] = tot;
+        if (threadIdx.x == 0) p.partials[member_off<BATCH>(p.pstride) + blockIdx.x] = tot;
     }
 }
 
@@ -283,33 +219,20 @@ static Plan plan_for(long n, long nrows, int K, int members = 0)
 }
 
 using PassKernel = void (*)(const Params);
-template <int ARITH>
+template <int ARITH, bool BATCH>
 static PassKernel pass_kernel_of(bool pre, int post)
 {
-    if (pre) return post == POST_NORM2 ? k_syst_pass<ARITH, true, POST_NORM2> : post == POST_INJECT ? k_syst_pass<ARITH, true, POST_INJECT>
-                                                                                                   : k_syst_pass<ARITH, true, POST_NONE>;
-    return post == POST_NORM2 ? k_syst_pass<ARITH, false, POST_NORM2> : post == POST_INJECT ? k_syst_pass<ARITH, false, POST_INJECT>
-                                                                                             : k_syst_pass<ARITH, false, POST_NONE>;
-}
-static PassKernel pass_kernel(int arith, bool pre, int post)
-{
     // full weighting: down leg only, no prolongation flavour
-    if (post == POST_FW) return arith == MGB200_ARITH_EXACT ? k_syst_pass<MGB200_ARITH_EXACT, false, POST_FW> : k_syst_pass<MGB200_ARITH_FAST, false, POST_FW>;
-    return arith == MGB200_ARITH_EXACT ? pass_kernel_of<MGB200_ARITH_EXACT>(pre, post) : pass_kernel_of<MGB200_ARITH_FAST>(pre, post);
+    if (post == POST_FW) return k_syst_pass<ARITH, false, POST_FW, BATCH>;
+    if (pre) return post == POST_NORM2 ? k_syst_pass<ARITH, true, POST_NORM2, BATCH> : post == POST_INJECT ? k_syst_pass<ARITH, true, POST_INJECT, BATCH>
+                                                                                                          : k_syst_pass<ARITH, true, POST_NONE, BATCH>;
+    return post == POST_NORM2 ? k_syst_pass<ARITH, false, POST_NORM2, BATCH> : post == POST_INJECT ? k_syst_pass<ARITH, false, POST_INJECT, BATCH>
+                                                                                                    : k_syst_pass<ARITH, false, POST_NONE, BATCH>;
 }
-
-template <int ARITH>
-static PassKernel batched_kernel_of(bool pre, int post)
+static PassKernel pass_kernel(int arith, bool pre, int post, bool batch)
 {
-    if (post == POST_FW) return k_syst_pass_batched<ARITH, false, POST_FW>;
-    if (pre) return post == POST_NORM2 ? k_syst_pass_batched<ARITH, true, POST_NORM2> : post == POST_INJECT ? k_syst_pass_batched<ARITH, true, POST_INJECT>
-                                                                                                           : k_syst_pass_batched<ARITH, true, POST_NONE>;
-    return post == POST_NORM2 ? k_syst_pass_batched<ARITH, false, POST_NORM2> : post == POST_INJECT ? k_syst_pass_batched<ARITH, false, POST_INJECT>
-                                                                                                     : k_syst_pass_batched<ARITH, false, POST_NONE>;
-}
-static PassKernel batched_kernel(int arith, bool pre, int post)
-{
-    return arith == MGB200_ARITH_EXACT ? batched_kernel_of<MGB200_ARITH_EXACT>(pre, post) : batched_kernel_of<MGB200_ARITH_FAST>(pre, post);
+    if (arith == MGB200_ARITH_EXACT) return batch ? pass_kernel_of<MGB200_ARITH_EXACT, true>(pre, post) : pass_kernel_of<MGB200_ARITH_EXACT, false>(pre, post);
+    return batch ? pass_kernel_of<MGB200_ARITH_FAST, true>(pre, post) : pass_kernel_of<MGB200_ARITH_FAST, false>(pre, post);
 }
 
 }  // namespace sy
@@ -326,18 +249,11 @@ int stream_pass_init()
     std::lock_guard<std::mutex> lock(mu);
     if (dev >= 0 && dev < 64 && done[dev]) return MGB200_OK;
     MGB_CUDA(cudaDeviceGetAttribute(&g_sms, cudaDevAttrMultiProcessorCount, dev));
-    for (int arith = 0; arith < 2; ++arith)
-        for (int pre = 0; pre < 2; ++pre)
-            for (int post = 0; post < 3; ++post)
-                MGB_CUDA(cudaFuncSetAttribute(pass_kernel(arith, pre != 0, post), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_BYTES));
-    for (int arith = 0; arith < 2; ++arith)
-        MGB_CUDA(cudaFuncSetAttribute(pass_kernel(arith, false, POST_FW), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_BYTES));
-    for (int arith = 0; arith < 2; ++arith) {
-        for (int pre = 0; pre < 2; ++pre)
-            for (int post = 0; post < 3; ++post)
-                MGB_CUDA(cudaFuncSetAttribute(batched_kernel(arith, pre != 0, post), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_BYTES));
-        MGB_CUDA(cudaFuncSetAttribute(batched_kernel(arith, false, POST_FW), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_BYTES));
-    }
+    for (int batch = 0; batch < 2; ++batch)
+        for (int arith = 0; arith < 2; ++arith)
+            for (int pre = 0; pre < 2; ++pre)
+                for (int post = 0; post <= POST_FW; ++post)
+                    MGB_CUDA(cudaFuncSetAttribute(pass_kernel(arith, pre != 0, post, batch != 0), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_BYTES));
     if (!g_encode) {
         void* fn = nullptr;
         cudaDriverEntryPointQueryResult qres;
@@ -373,7 +289,7 @@ static int build_params(const StreamPassArgs& a, Params& p, unsigned& grid_out, 
     const long own_lo = whole ? 0 : a.own_lo, own_hi = whole ? a.n : a.own_hi;
     if (a.members < 0 || a.members > STREAM_PASS_MAX_MEMBERS) return fail(MGB200_ERR_INVALID, "stream_pass: members must be 0..65535");
     const bool batch = a.members > 0;
-    if (batch && (!whole || !a.active || a.mstride <= 0 || (a.coarse_u && a.cmstride <= 0) || a.sync))
+    if (batch && (!whole || !a.active || a.mstride <= 0 || (a.coarse_u && a.cmstride <= 0)))
         return fail(MGB200_ERR_INVALID, "stream_pass: a batched pass needs whole levels, member strides and the active flags");
     const Plan pl = plan_for(a.n, own_hi - own_lo + 1, a.iters, a.members);
     p = Params{};
@@ -390,7 +306,6 @@ static int build_params(const StreamPassArgs& a, Params& p, unsigned& grid_out, 
     p.post = a.post;
     p.u_is_zero = a.u_in ? 0 : 1;
     p.CW = pl.SWK / 2 + 8;
-    { const char* e = getenv("MGB200_SY_BACKOFF"); p.backoff_ns = e ? atoi(e) : 0; }   // tuning aid
     p.st = a.st;
     p.u_in = a.u_in; p.rhs = a.rhs; p.v1 = a.v1; p.v2 = a.v2; p.cu = a.coarse_u;
     // the u map of a zero-input pass is never dereferenced (its boxes lie out of bounds): any valid field will do
@@ -402,9 +317,6 @@ static int build_params(const StreamPassArgs& a, Params& p, unsigned& grid_out, 
     if (a.coarse_u) MGB_TRY(encode_field(&p.maps[FIELD_C], a.coarse_u, a.Lc.odd, a.Lc.pitch, p.crows_mem, p.CW, CROWS, mb, a.cmstride));
     p.u_out = a.u_out; p.crhs = a.coarse_rhs; p.partials = a.partials;
     if (batch) { p.mstride = a.mstride; p.cmstride = a.cmstride; p.pstride = a.pstride; p.active = a.active; }
-    p.peer_u_up = a.peer_u_up; p.peer_u_dn = a.peer_u_dn; p.peer_c_up = a.peer_c_up; p.peer_c_dn = a.peer_c_dn;
-    p.push_rows = a.push_rows; p.c_own_lo = a.c_own_lo; p.c_own_hi = a.c_own_hi;
-    p.sync = a.sync; p.raise_up = a.raise_up; p.raise_dn = a.raise_dn;
     if (p.post == POST_INJECT && !p.crhs) return fail(MGB200_ERR_INVALID, "stream_pass: POST_INJECT without coarse_rhs");
     if (p.post == POST_FW && (!p.crhs || p.pre)) return fail(MGB200_ERR_INVALID, "stream_pass: POST_FW needs coarse_rhs and no prolongation");
     if (p.post == POST_NORM2 && !p.partials) return fail(MGB200_ERR_INVALID, "stream_pass: POST_NORM2 without partials");
@@ -432,9 +344,6 @@ int stream_pass(const StreamPassArgs& a, cudaStream_t s)
         key.iters = a.iters; key.coarse_u = a.coarse_u; key.Lc = a.Lc; key.post = a.post; key.coarse_rhs = a.coarse_rhs;
         key.partials = a.partials; key.arith = a.arith; key.own_lo = a.own_lo; key.own_hi = a.own_hi; key.row0 = a.row0;
         key.rows_mem = a.rows_mem; key.crow0 = a.crow0; key.crows_mem = a.crows_mem;
-        key.peer_u_up = a.peer_u_up; key.peer_u_dn = a.peer_u_dn; key.peer_c_up = a.peer_c_up; key.peer_c_dn = a.peer_c_dn;
-        key.push_rows = a.push_rows; key.c_own_lo = a.c_own_lo; key.c_own_hi = a.c_own_hi; key.sync = a.sync;
-        key.raise_up = a.raise_up; key.raise_dn = a.raise_dn;
         key.members = a.members; key.mstride = a.mstride; key.cmstride = a.cmstride; key.pstride = a.pstride; key.active = a.active;
         std::string k(reinterpret_cast<const char*>(&key), sizeof(key));
         auto it = cache.find(k);
@@ -447,11 +356,8 @@ int stream_pass(const StreamPassArgs& a, cudaStream_t s)
         }
         e = it->second;                                 // copied under the lock: the map may be cleared by another thread
     }
-    if (e.members > 0) {
-        batched_kernel(a.arith, e.p.pre != 0, e.p.post)<<<dim3(e.grid, (unsigned)e.members), THREADS, e.smem, s>>>(e.p);
-        return check_launch("k_syst_pass_batched");
-    }
-    pass_kernel(a.arith, e.p.pre != 0, e.p.post)<<<e.grid, THREADS, e.smem, s>>>(e.p);
+    const bool batch = e.members > 0;
+    pass_kernel(a.arith, e.p.pre != 0, e.p.post, batch)<<<dim3(e.grid, batch ? (unsigned)e.members : 1u), THREADS, e.smem, s>>>(e.p);
     return check_launch("k_syst_pass");
 }
 

@@ -90,7 +90,6 @@ struct Params {
     int post;                  // StreamPost
     int u_is_zero;             // u_in == 0 everywhere: rows are zero-filled by an out-of-bounds box
     int CW;                    // SWK/2 + 8: coarse pairs per smem run
-    int backoff_ns;            // pause between two unsuccessful looks at a progress counter (0: none)
     Stencil st;
     const double* u_in;
     const double* rhs;
@@ -100,11 +99,7 @@ struct Params {
     double* u_out;
     double* crhs;              // coarse rhs (POST_INJECT, POST_FW)
     double* partials;          // POST_NORM2
-    // halo push fused into the pass (stream_pass.cuh); peer_* are addressed by GLOBAL row: peer + row * pitch
-    double* peer_u_up; double* peer_u_dn; double* peer_c_up; double* peer_c_dn;
-    long push_rows, c_own_lo, c_own_hi;
-    int* sync; int* raise_up; int* raise_dn;
-    // batched passes (k_syst_pass_batched): member b of every fine / coarse array starts b * mstride / b * cmstride
+    // batched passes (BATCH): member b of every fine / coarse array starts b * mstride / b * cmstride
     // doubles after the first, its partial sums at b * pstride; a member whose active[b] is 0 is not touched
     long mstride, cmstride, pstride;
     const int* active;
@@ -193,10 +188,9 @@ SY_FN void sy_full_wait(const Smem& sm, int g, unsigned parity);
 struct Prog2 { unsigned h0, h1; };
 SY_FN void sy_prog_publish(const Smem& sm, int warp, unsigned steps_done);
 SY_FN Prog2 sy_prog_peek(const Smem& sm, int stage);
-SY_FN void sy_backoff(int ns);                           // between two unsuccessful peeks
-// row slabs: wait until arrival counter `slot` of the block `sync` has reached the number of passes this rank has
-// completed (one thread)
-SY_FN void sy_wait_neighbour(int* sync, int slot);
+// between two unsuccessful peeks at the counters of pair `pair`: nothing on the device; the host model yields there
+// and reports a deadlock
+SY_FN void sy_backoff(int pair);
 SY_FN void sy_bulk_store(const Smem& sm, double* gdst, unsigned soff, unsigned bytes);
 SY_FN void sy_store_commit();
 SY_FN void sy_store_wait_read0();                        // every committed store has read its shared memory
@@ -222,7 +216,6 @@ struct Geo {
     unsigned cwb;     // bytes of one coarse parity run
     unsigned cgrpb;   // bytes of the coarse rows of one group
     int nh;           // warps per stage that hold live pairs (1 for strips of <= 64 pairs)
-    int backoff_ns;
 };
 SY_FN Geo make_geo(const Params& p)
 {
@@ -230,7 +223,6 @@ SY_FN Geo make_geo(const Params& p)
     g.swkb = (unsigned)p.SWK * 8u; g.rowb = 2u * g.swkb; g.ringb = (unsigned)RING * g.rowb;
     g.cwb = (unsigned)p.CW * 8u; g.cgrpb = (unsigned)CROWS * 2u * g.cwb;
     g.nh = p.SWK > 64 ? 2 : 1;
-    g.backoff_ns = p.backoff_ns;
     return g;
 }
 
@@ -335,9 +327,9 @@ SY_FN void advance_row(const Geo& geo, Stage& st)
 }
 
 // wait until the warps of pair `pair` have completed `need0` / `need1` steps (pv: a peek taken earlier)
-SY_FN void prog_wait(const Smem& sm, int pair, unsigned need0, unsigned need1, Prog2 pv, int backoff_ns = 0)
+SY_FN void prog_wait(const Smem& sm, int pair, unsigned need0, unsigned need1, Prog2 pv)
 {
-    while (pv.h0 < need0 || pv.h1 < need1) { sy_backoff(backoff_ns); pv = sy_prog_peek(sm, pair); }
+    while (pv.h0 < need0 || pv.h1 < need1) { sy_backoff(pair); pv = sy_prog_peek(sm, pair); }
 }
 
 // wait for the data of step k: the TMA group of row t (roles fed by the TMA engine) or step k-1 of the role above
@@ -350,7 +342,7 @@ SY_FN void wait_inputs(const Tile& tl, const Geo& geo, const Smem& sm, const Sta
             sy_full_wait(sm, g % NGROUP, (unsigned)(g / NGROUP) & 1u);
         }
     } else {
-        prog_wait(sm, st.up, (unsigned)k, geo.nh == 2 ? (unsigned)k : 0u, seen, geo.backoff_ns);
+        prog_wait(sm, st.up, (unsigned)k, geo.nh == 2 ? (unsigned)k : 0u, seen);
     }
 }
 
@@ -410,24 +402,13 @@ SY_FN void pre_loop(const Params& p, const Tile& tl, const Geo& geo, const Smem&
 
 // ------------------------------------------------------------------------------------------
 // Coarse right-hand side node pair (cr, kg), (cr, kg+1) of a lane whose vector starts at global pair kg (even: the
-// strips start at even pairs): kg -> E run at kg/2, kg+1 -> O run; only the owned interior columns (rmask0), and
-// the same values into the slab neighbours' halo rows of the coarse rhs.
+// strips start at even pairs): kg -> E run at kg/2, kg+1 -> O run; only the owned interior columns (rmask0).
 template <bool BATCH>
 SY_FN void store_coarse(const Params& p, const Stage& st, long kg, long cr, double r0, double r1)
 {
     double* crow = p.crhs + member_off<BATCH>(p.cmstride) + (cr - p.crow0) * p.cpitch + (kg >> 1);
     if (st.rmask0 & 1u) crow[0] = r0;
     if (st.rmask0 & 2u) crow[p.codd] = r1;
-    if (p.peer_c_up && cr < p.c_own_lo + p.push_rows) {
-        double* q = p.peer_c_up + cr * p.cpitch + (kg >> 1);
-        if (st.rmask0 & 1u) q[0] = r0;
-        if (st.rmask0 & 2u) q[p.codd] = r1;
-    }
-    if (p.peer_c_dn && cr > p.c_own_hi - p.push_rows) {
-        double* q = p.peer_c_dn + cr * p.cpitch + (kg >> 1);
-        if (st.rmask0 & 1u) q[0] = r0;
-        if (st.rmask0 & 2u) q[p.codd] = r1;
-    }
 }
 
 // POST_FW: byte offset of node kk of residual row `row` (E run; the O run follows at + swkb)
@@ -451,7 +432,7 @@ template <bool BATCH>
 SY_FN void fw_restrict_row(const Params& p, const Tile& tl, const Geo& geo, const Smem& sm, const Stage& st, FwSums& fw,
                            const int k, const int q, const bool live)
 {
-    prog_wait(sm, PAIR_EPI, (unsigned)k, geo.nh == 2 ? (unsigned)k : 0u, sy_prog_peek(sm, PAIR_EPI), geo.backoff_ns);
+    prog_wait(sm, PAIR_EPI, (unsigned)k, geo.nh == 2 ? (unsigned)k : 0u, sy_prog_peek(sm, PAIR_EPI));
     const unsigned b = fw_off(tl, geo, st, q);
     D2 e{0.0, 0.0}, o{0.0, 0.0};
     if (live) { e = sy_lds2(sm, b); o = sy_lds2(sm, b + geo.swkb); }
@@ -538,7 +519,7 @@ SY_FN void stage_step(const Params& p, const Tile& tl, const Geo& geo, const Sme
             // both have published their step on row - FW_ROWS + 2 (they restrict row q after publishing row q + 1):
             // EPI step k + 5 - FW_ROWS (its rows trail this stage's by 2)
             const int need = k + 5 - FW_ROWS;
-            if (need > 0) prog_wait(sm, PAIR_EPI, (unsigned)need, geo.nh == 2 ? (unsigned)need : 0u, seen_epi, geo.backoff_ns);
+            if (need > 0) prog_wait(sm, PAIR_EPI, (unsigned)need, geo.nh == 2 ? (unsigned)need : 0u, seen_epi);
             const double r0 = Arith<ARITH>::residual(f.x, o0, up.x, n0, dn.x, n1, c0, p.st);
             const double r1 = Arith<ARITH>::residual(f.y, o1, up.y, n1, dn.y, n2, c1, p.st);
             if (live) sy_sts2(sm, fw_off(tl, geo, st, row) + po, D2{r0, r1});
@@ -690,7 +671,6 @@ SY_FN void store_loop(const Params& p, const Tile& tl, const Geo& geo, const Sme
     unsigned a = (unsigned)((((rs - tl.R0) % RING) + RING) % RING) * geo.rowb + (unsigned)HK * 8u;
     const unsigned awrap = geo.ringb + (unsigned)HK * 8u;
     const unsigned need_h1 = geo.nh == 2 ? 1u : 0u;
-    const bool push = p.peer_u_up != nullptr || p.peer_u_dn != nullptr;
     Prog2 seen_s{0u, 0u};
     unsigned groups = 0;
     for (int k = 0; k <= klast; ++k, ++rs) {
@@ -700,7 +680,7 @@ SY_FN void store_loop(const Params& p, const Tile& tl, const Geo& geo, const Sme
         // last do not cover this row)
         if ((store || close) && (seen_s.h0 < (unsigned)k + 1u || seen_s.h1 < need_h1 * ((unsigned)k + 1u))) {
             seen_s = sy_prog_peek(sm, pair_s);
-            while (seen_s.h0 < (unsigned)k + 1u || seen_s.h1 < need_h1 * ((unsigned)k + 1u)) { sy_backoff(geo.backoff_ns); seen_s = sy_prog_peek(sm, pair_s); }
+            while (seen_s.h0 < (unsigned)k + 1u || seen_s.h1 < need_h1 * ((unsigned)k + 1u)) { sy_backoff(pair_s); seen_s = sy_prog_peek(sm, pair_s); }
         }
         if (close) ++groups;
         if ((store || close) && sy_elect()) {
@@ -708,20 +688,6 @@ SY_FN void store_loop(const Params& p, const Tile& tl, const Geo& geo, const Sme
                 sy_fence_async();                                    // the stages' stores (acquired above) -> the engine's reads
                 if (nE8) sy_bulk_store(sm, gstE, a, nE8);
                 if (nO8) sy_bulk_store(sm, gstO, a + geo.swkb, nO8);
-                // row slabs: the first / last rows this rank produces are the neighbours' halo rows: the same bulk
-                // copies, addressed to their memory (NVLink peer mapping), in the same group
-                if (push) {
-                    if (p.peer_u_up && rs < p.own_lo + p.push_rows) {
-                        double* q = p.peer_u_up + (long)rs * pitch + tl.kb;
-                        if (nE8) sy_bulk_store(sm, q, a, nE8);
-                        if (nO8) sy_bulk_store(sm, q + p.odd, a + geo.swkb, nO8);
-                    }
-                    if (p.peer_u_dn && rs > p.own_hi - p.push_rows) {
-                        double* q = p.peer_u_dn + (long)rs * pitch + tl.kb;
-                        if (nE8) sy_bulk_store(sm, q, a, nE8);
-                        if (nO8) sy_bulk_store(sm, q + p.odd, a + geo.swkb, nO8);
-                    }
-                }
             }
             if (close) {
                 sy_store_commit();

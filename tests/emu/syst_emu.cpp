@@ -124,18 +124,17 @@ SY_FN Prog2 sy_prog_peek(const Smem&, int stage)
     v.h1 = g_prog[2 * stage + 1].load(std::memory_order_acquire);
     return v;
 }
-SY_FN void sy_backoff(int)
+SY_FN void sy_backoff(int pair)
 {
     static thread_local long spins = 0;
     sched_yield();
     if (++spins % 3000000L == 0) {                        // a protocol deadlock: die loudly instead of hanging the suite
-        std::fprintf(stderr, "syst_emu: warp %d lane %d has been spinning on a progress counter; steps published:", t_warp, t_lane);
+        std::fprintf(stderr, "syst_emu: warp %d lane %d has been spinning on the progress counters of pair %d; steps published:", t_warp, t_lane, pair);
         for (int w = 0; w < NSTAGE; ++w) std::fprintf(stderr, " %ld", g_done[w].load());
         std::fprintf(stderr, "\n");
         std::abort();
     }
 }
-SY_FN void sy_wait_neighbour(int*, int) {}
 SY_FN void sy_bulk_store(const Smem& sm, double* gdst, unsigned soff, unsigned bytes) { std::memcpy(gdst, sm.raw + soff, bytes); }
 SY_FN void sy_store_commit() {}
 SY_FN void sy_store_wait_read0() {}

@@ -1,5 +1,5 @@
 // syst_emu_batched.cpp -- TEST INFRASTRUCTURE: the host model of the streaming kernel (syst_emu_fw.cpp, which
-// includes syst_emu.cpp) extended by the batched flavour (k_syst_pass_batched): `members` problems of one size,
+// includes syst_emu.cpp) extended by the batched flavour (k_syst_pass with BATCH = true): `members` problems of one size,
 // member b of every fine / coarse array b * mstride / b * cmstride doubles after the first, tile t of member b run
 // with sy_member() = b.  A member whose active flag is 0 is skipped whole, as the kernel's blocks return before they
 // touch anything.  The 4-D tensor copy zero-fills outside the member's rows.  Also exports make_plan.  Never linked
